@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- match-search throughput of sqz-b200 on B200, beside the reference CPU codec.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size BYTES]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size BYTES] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[4], SURVEY.md section 8d config 5): the 1 GiB synthetic corpus
@@ -209,6 +209,28 @@ def workload_config(args) -> dict:
     }
 
 
+def dump_outputs(path: str, d_table, d_tokens) -> None:
+    """What the last timed step handed its caller, as .npy files: the match table of rank 0's shard
+    (length and distance per position) and the whole token stream.  Both are far larger than 64 MB,
+    so fixed seeded samples of positions are written, with the positions themselves; the values are
+    exact in float32 (16-bit length and distance) and float64 (32-bit tokens, positions)."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0x53515A)
+
+    def sample(n: int, k: int) -> np.ndarray:
+        return np.arange(n) if n <= k else np.unique(rng.integers(0, n, k))
+
+    pos = sample(d_table.numel(), 2 << 20)
+    w = d_table[torch.from_numpy(pos).to(d_table.device)].cpu().numpy().view(np.uint32)
+    at = sample(d_tokens.numel(), 1 << 20)
+    tok = d_tokens[torch.from_numpy(at).to(d_tokens.device)].cpu().numpy().view(np.uint32)
+    for name, a in (("match_position", pos.astype(np.float64)), ("match_len", (w >> 16).astype(np.float32)),
+                    ("match_dist", (w & 0xFFFF).astype(np.float32)), ("token_index", at.astype(np.float64)),
+                    ("token", tok.astype(np.float64)), ("token_count", np.array([d_tokens.numel()], np.float64))):
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- our arm
 class DeviceArray:
     """A raw device allocation of the library seen as a CUDA array (torch.as_tensor wraps it)."""
@@ -392,6 +414,14 @@ def ours(args) -> None:
     n_tokens = sum_over_ranks(n_tokens_mine)
     launches = sum_over_ranks(leg["launches"])
     t_match_max = max_over_ranks(t_match)
+    if args.dump_outputs and rank == 0:
+        if world == 1:
+            toks = leg["d_tokens"][:n_tokens]
+        elif gather_ptr:
+            toks = torch.as_tensor(DeviceArray(gather_ptr, n_tokens), device=dev)
+        else:
+            raise SystemExit("--dump-outputs: the token stream was not gathered on GPU 0")
+        dump_outputs(args.dump_outputs, d_table, toks)
 
     # visited candidate-compares: what the reference's scan really walks (it stops at the nearest
     # max_len candidate, squeeze.h:353); algorithmic CC ignores that early-out (SURVEY 8d)
@@ -759,7 +789,11 @@ def main():
     ap.add_argument("--kind-bytes", type=int, default=64 << 20, help="bytes per kind of the per_kind table (N = 1); 0 = skip")
     ap.add_argument("--cpu-sample", type=int, default=512 << 10)
     ap.add_argument("--compress-sample", type=int, default=256 << 20)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write samples of the last timed step's match table and token stream to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         reference_arm(args)
     else:
