@@ -7,8 +7,10 @@
  * maintainer would call at exactly that place (see INTEGRATION.md): plain
  * pointers and sizes, int errno return values, callable from C99.  No call
  * changes the calling thread's current CUDA device.  State that outlives a call
- * is limited to recycled staging buffers (sqz_gpu_release frees them) and the
- * measurement aids at the end of this file, which are off unless switched on.
+ * is limited to staging buffers kept for the next call -- per device at most 8
+ * sets and 12 GiB of device + pinned memory, oldest out first; sqz_gpu_release
+ * frees them -- and the measurement aids at the end of this file, which are off
+ * unless switched on.
  *
  * Rule parameters (SURVEY.md section 8a, row A1):
  *   window    the LZ window the stream header announces (power of two)
@@ -214,9 +216,10 @@ int         sqz_gpu_device_count(void);          /* 0 when no driver / device */
 const char* sqz_gpu_last_error(void);            /* thread-local text */
 void*       sqz_gpu_host_alloc(size_t bytes);    /* pinned host memory (NULL on failure) */
 void        sqz_gpu_host_free(void* p);
-/* The host-buffer entry points keep their device and pinned staging buffers
- * for the next call (at most four slots and 3 GiB, oldest out first), and the
- * plain device entry point keeps its scratch buffers; this frees them all.   */
+/* The host-buffer entry points and sqz_gpu_match_table_device keep their device
+ * and pinned staging buffers for the next call: one set per shard or pipeline
+ * slot, per device at most 8 sets and 12 GiB of device + pinned memory, oldest
+ * out first.  This frees them all.                                           */
 void        sqz_gpu_release(void);
 /* Which match-table kernel serves sqz_gpu_match_table_device: 0 = automatic
  * (bit-sliced kernel for min_len 2 or 3, thread-per-position kernel otherwise),

@@ -608,7 +608,7 @@ struct ScopedEvent {
 // ---------------------------------------------------------------------------
 // workspace of the match table: the segment cursor of phase 2 and phase 1's work list
 // (one bit per position).  Callers of the _ws entry point own it; the plain entry point
-// borrows one from a small per-device pool and hands it back when the stream has passed.
+// borrows a parked one (a kWorkspace stage, below) and gives it back on the caller's stream.
 // ---------------------------------------------------------------------------
 constexpr size_t kCursorBytes = 256;
 
@@ -672,69 +672,188 @@ extern "C" size_t sqz_gpu_match_workspace(size_t n) {
     return kCursorBytes + mask_bytes(n) + tables;
 }
 
-struct PoolBuffer { void* ptr; size_t bytes; cudaEvent_t passed; int device; };
-static std::mutex g_pool_mu;
-static std::vector<PoolBuffer> g_pool;          // idle or in flight (passed not yet reached)
-constexpr size_t kPoolMax = 16;
+// ---------------------------------------------------------------------------
+// staging buffers, kept between calls
+// ---------------------------------------------------------------------------
 
-static int pool_take(size_t bytes, PoolBuffer* out) {
-    int dev = 0;
-    CU(cudaGetDevice(&dev));
-    {
-        std::lock_guard<std::mutex> lk(g_pool_mu);
-        for (size_t k = 0; k < g_pool.size(); k++) {
-            PoolBuffer& b = g_pool[k];
-            if (b.device == dev && b.bytes >= bytes && b.bytes <= 4 * bytes + (1u << 20) &&
-                cudaEventQuery(b.passed) == cudaSuccess) {
-                *out = b;
-                g_pool.erase(g_pool.begin() + (long)k);
-                return 0;
-            }
-        }
-        cudaGetLastError();                      // cudaErrorNotReady of a busy buffer is not an error
+// the calling thread's current device is the caller's business: every entry point that has to
+// switch (an explicit stream device, the multi-device call) puts it back on the way out
+struct DeviceScope {
+    int saved = -1;
+    DeviceScope() { if (cudaGetDevice(&saved) != cudaSuccess) { saved = -1; cudaGetLastError(); } }
+    ~DeviceScope() { if (saved >= 0) { cudaSetDevice(saved); } }
+};
+
+// What a stage holds depends on what its user needs:
+//   kWorkspace  the match workspace only: sqz_gpu_match_table_device borrows it on the caller's stream.
+//   the others  the workspace, a stream of their own, the shard with its halos (sized for the library's
+//               limits), its match table, the parse result (device and pinned) and the events, and
+//     kTable    the table's two 16-bit halves (sqz_gpu_match_table);
+//     kTokens   the tokens, the parse workspace and the exit map (sqz_gpu_tokens, sqz_gpu_tokens_multi);
+//     kConsumer kTokens plus pinned tokens and a stream of the highest priority (sqz_gpu_stream_*).
+enum { kWorkspace, kTable, kTokens, kConsumer };
+
+// the buffers and streams for one shard of at most `cap` positions on one device
+struct Stage {
+    int device = -1, kind = kWorkspace;
+    size_t cap = 0;
+    size_t bytes = 0;                 // device + pinned memory it holds
+    cudaEvent_t idle = nullptr;       // all its work is over (recorded when it is given back)
+    void* d_mwork = nullptr;          // match workspace (cursor + work list of phase 2)
+    cudaStream_t stream = nullptr;
+    cudaStream_t ahead_of_all = nullptr;   // highest priority: a consumer's parse and token copy
+    cudaEvent_t done = nullptr;       // everything of the chunk has been issued and finished
+    cudaEvent_t parsed = nullptr;     // the chunk's token count and overshoot are in h_result
+    cudaEvent_t tabled = nullptr;     // the match table is complete (multi-device call: its exit map is in h_map)
+    uint8_t* d_data = nullptr;        // back halo + shard + ahead halo
+    uint32_t* d_table = nullptr;
+    uint64_t* d_result = nullptr;     // [0] tokens, [1] overshoot (next shard's entry)
+    uint64_t* h_result = nullptr;     // pinned
+    uint16_t* d_len = nullptr;
+    uint16_t* d_dist = nullptr;
+    uint32_t* d_tokens = nullptr;
+    void* d_work = nullptr;           // parse workspace
+    uint16_t* d_map = nullptr;        // exit map
+    uint16_t* h_map = nullptr;        // pinned
+    uint32_t* h_tokens = nullptr;     // pinned
+    size_t first = 0, n = 0, back = 0;     // the shard it holds: [first, first + n) of the input
+    bool busy = false;
+};
+
+// on the current device, which is s.device
+static int stage_alloc(Stage& s) {
+    auto dev = [&s](auto** p, size_t b) { s.bytes += b; return cudaMalloc(p, b); };
+    auto pin = [&s](auto** p, size_t b) { s.bytes += b; return cudaHostAlloc(p, b, cudaHostAllocDefault); };
+    CU(cudaEventCreateWithFlags(&s.idle, cudaEventDisableTiming));
+    CU(dev(&s.d_mwork, sqz_gpu_match_workspace(s.cap)));
+    if (s.kind == kWorkspace) { return 0; }
+    CU(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
+    CU(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&s.parsed, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&s.tabled, cudaEventDisableTiming));
+    CU(dev(&s.d_data, (size_t)sqz_gpu_max_dist_limit + s.cap + sqz_gpu_max_len_limit + 64));
+    CU(dev(&s.d_table, s.cap * 4));
+    CU(dev(&s.d_result, 16));
+    CU(pin(&s.h_result, 16));
+    if (s.kind == kTable) {
+        CU(dev(&s.d_len, s.cap * 2));
+        CU(dev(&s.d_dist, s.cap * 2));
+        return 0;
     }
-    PoolBuffer b{nullptr, bytes, nullptr, dev};
-    CU(cudaMalloc(&b.ptr, bytes));
-    cudaError_t ce = cudaEventCreateWithFlags(&b.passed, cudaEventDisableTiming);
-    if (ce != cudaSuccess) { cudaFree(b.ptr); return fail(cuda_code(ce), "cudaEventCreate", ce); }
-    *out = b;
+    CU(dev(&s.d_tokens, s.cap * 4 + 16));
+    CU(dev(&s.d_work, parse::workspace(s.cap)));
+    CU(dev(&s.d_map, parse::kMapStride * 2));
+    CU(pin(&s.h_map, parse::kMapStride * 2));
+    if (s.kind == kConsumer) {
+        CU(pin(&s.h_tokens, s.cap * 4 + 16));
+        int least = 0, greatest = 0;
+        CU(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        CU(cudaStreamCreateWithPriority(&s.ahead_of_all, cudaStreamNonBlocking, greatest));
+    }
     return 0;
 }
 
-static void pool_free(PoolBuffer& b) {
-    cudaEventSynchronize(b.passed);
-    cudaEventDestroy(b.passed);
-    cudaFree(b.ptr);
+static void stage_free(Stage& s) {
+    DeviceScope keep;
+    cudaSetDevice(s.device);
+    if (s.idle) { cudaEventSynchronize(s.idle); }
+    if (s.stream) { cudaStreamSynchronize(s.stream); }
+    if (s.ahead_of_all) { cudaStreamSynchronize(s.ahead_of_all); }
+    cudaFree(s.d_mwork); cudaFree(s.d_data); cudaFree(s.d_table); cudaFree(s.d_result); cudaFree(s.d_len);
+    cudaFree(s.d_dist); cudaFree(s.d_tokens); cudaFree(s.d_work); cudaFree(s.d_map);
+    cudaFreeHost(s.h_result); cudaFreeHost(s.h_map); cudaFreeHost(s.h_tokens);
+    for (cudaEvent_t e : {s.idle, s.done, s.parsed, s.tabled}) { if (e) { cudaEventDestroy(e); } }
+    for (cudaStream_t q : {s.stream, s.ahead_of_all}) { if (q) { cudaStreamDestroy(q); } }
+    s = Stage();
 }
 
-// the work queued on `s` so far is the last user of the buffer
-static void pool_give_back(PoolBuffer b, cudaStream_t s) {
-    cudaEventRecord(b.passed, s);
-    PoolBuffer victim{nullptr, 0, nullptr, 0};
+// Allocating and freeing gigabytes of device and pinned memory per call costs more than the search of
+// a small input and stalls the device: finished calls park their stages here, and a later call takes
+// back one of the same device and kind that is large enough and at most four times too large.  Per
+// device at most kParkStages stages and kParkBytes of device + pinned memory stay parked, oldest out
+// first (a 512 MiB shard of sqz_gpu_tokens_multi holds about 4.7 GiB); sqz_gpu_release() frees them.
+static std::mutex g_park_mu;
+static std::vector<Stage> g_park;                 // oldest first
+constexpr size_t kParkStages = 8;
+constexpr size_t kParkBytes = (size_t)12 << 30;
+
+// a stage of this kind for n positions on `device`, which is the current device
+static int stage_take(Stage& s, int device, int kind, size_t n) {
+    size_t cap = (size_t)1 << 20;            // a power of two (>= 1 Mi) so that calls of similar size share stages
+    while (cap < n) { cap <<= 1; }
     {
-        std::lock_guard<std::mutex> lk(g_pool_mu);
-        g_pool.push_back(b);
-        if (g_pool.size() > kPoolMax) { victim = g_pool.front(); g_pool.erase(g_pool.begin()); }
+        std::lock_guard<std::mutex> lk(g_park_mu);
+        for (size_t k = 0; k < g_park.size(); k++) {
+            const Stage& c = g_park[k];
+            if (c.device == device && c.kind == kind && c.cap >= cap && c.cap <= 4 * cap &&
+                cudaEventQuery(c.idle) == cudaSuccess) {
+                s = c;
+                s.busy = false;
+                g_park.erase(g_park.begin() + (long)k);
+                return 0;
+            }
+        }
+        cudaGetLastError();                  // cudaErrorNotReady of a stage still in use is not an error
     }
-    if (victim.ptr != nullptr) {
-        int cur = 0;
-        cudaGetDevice(&cur);
-        cudaSetDevice(victim.device);
-        pool_free(victim);
-        cudaSetDevice(cur);
-    }
+    s = Stage();
+    s.device = device;
+    s.kind = kind;
+    s.cap = cap;
+    const int r = stage_alloc(s);
+    if (r != 0) { stage_free(s); }
+    return r;
 }
 
-static void pool_release_all() {
-    std::vector<PoolBuffer> all;
+// parks a stage whose work so far is all joined into `q`
+static void stage_give_back(Stage& s, cudaStream_t q) {
+    if (s.idle == nullptr) { return; }       // never allocated
+    cudaError_t ce;
     {
-        std::lock_guard<std::mutex> lk(g_pool_mu);
-        all.swap(g_pool);
+        DeviceScope keep;
+        cudaSetDevice(s.device);
+        ce = cudaEventRecord(s.idle, q);
     }
-    int cur = 0;
-    cudaGetDevice(&cur);
-    for (PoolBuffer& b : all) { cudaSetDevice(b.device); pool_free(b); }
-    cudaSetDevice(cur);
+    // not kept: a stage without its idle mark, and one above the bound on its own (it would only push
+    // the others out)
+    std::vector<Stage> victims;
+    if (ce != cudaSuccess || s.bytes > kParkBytes) {
+        victims.push_back(s);
+    } else {
+        std::lock_guard<std::mutex> lk(g_park_mu);
+        g_park.push_back(s);
+        size_t count = 0, bytes = 0;
+        for (const Stage& c : g_park) {
+            if (c.device == s.device) { count++; bytes += c.bytes; }
+        }
+        for (size_t k = 0; k < g_park.size() && (count > kParkStages || bytes > kParkBytes);) {
+            if (g_park[k].device != s.device) { k++; continue; }
+            count--;
+            bytes -= g_park[k].bytes;
+            victims.push_back(g_park[k]);
+            g_park.erase(g_park.begin() + (long)k);
+        }
+    }
+    s = Stage();
+    for (Stage& v : victims) { stage_free(v); }
+}
+
+// waits for the stage's stream and parks the stage; returns rc, or the wait's error when rc is 0
+static int stage_finish(Stage& s, int rc) {
+    if (s.stream != nullptr) {
+        const cudaError_t ce = cudaStreamSynchronize(s.stream);
+        if (ce != cudaSuccess && rc == 0) { rc = fail(cuda_code(ce), "cudaStreamSynchronize", ce); }
+    }
+    stage_give_back(s, s.stream);
+    return rc;
+}
+
+extern "C" void sqz_gpu_release(void) {
+    std::vector<Stage> all;
+    {
+        std::lock_guard<std::mutex> lk(g_park_mu);
+        all.swap(g_park);
+    }
+    for (Stage& s : all) { stage_free(s); }
 }
 
 static int launch_v1(const uint8_t* d_shard, size_t back, size_t n, size_t ahead, uint32_t min_len,
@@ -885,10 +1004,12 @@ extern "C" int sqz_gpu_match_table_device(const uint8_t* d_shard, size_t back, s
                                           uint32_t max_dist, uint32_t* d_table, void* stream) {
     if (int r = check_rules(min_len, max_len, max_dist)) { return r; }
     if (n == 0) { return 0; }
-    PoolBuffer b;
-    if (int r = pool_take(sqz_gpu_match_workspace(n), &b)) { return r; }
-    const int r = sqz_gpu_match_table_device_ws(d_shard, back, n, ahead, min_len, max_len, max_dist, d_table, b.ptr, stream);
-    pool_give_back(b, (cudaStream_t)stream);
+    int dev = 0;
+    CU(cudaGetDevice(&dev));
+    Stage w;
+    if (int r = stage_take(w, dev, kWorkspace, n)) { return r; }
+    const int r = sqz_gpu_match_table_device_ws(d_shard, back, n, ahead, min_len, max_len, max_dist, d_table, w.d_mwork, stream);
+    stage_give_back(w, (cudaStream_t)stream);
     return r;
 }
 
@@ -1025,34 +1146,6 @@ tokens_to_host(const uint32_t* __restrict__ d_tokens, const uint64_t* __restrict
     }
 }
 
-struct Slot {
-    cudaStream_t stream = nullptr;
-    cudaStream_t ahead_of_all = nullptr;   // highest priority: a consumer's parse and token copy (kModeTokensPinned)
-    cudaEvent_t done = nullptr;       // everything of the chunk has been issued and finished
-    cudaEvent_t parsed = nullptr;     // the chunk's token count and overshoot are in h_result
-    cudaEvent_t tabled = nullptr;     // the chunk's match table is complete
-    uint8_t* d_data = nullptr;        // back halo + chunk + ahead halo
-    uint32_t* d_table = nullptr;
-    uint32_t* d_tokens = nullptr;
-    uint16_t* d_len = nullptr;        // table mode only
-    uint16_t* d_dist = nullptr;
-    void* d_work = nullptr;           // parse workspace
-    void* d_mwork = nullptr;          // match workspace (cursor + work list of phase 2)
-    uint64_t* d_result = nullptr;     // [0] tokens, [1] overshoot (next chunk's entry)
-    uint64_t* h_result = nullptr;     // pinned
-    uint32_t* h_tokens = nullptr;     // pinned (streaming consumers only)
-    size_t first = 0, n = 0;          // chunk = [first, first + n) of the input
-    bool busy = false;
-    // what the buffers were sized for (slots are recycled between calls, see slot_take)
-    int device = -1;
-    size_t cap_chunk = 0;
-    uint32_t cap_len = 0, cap_dist = 0;
-    int cap_mode = 0;
-    size_t device_bytes = 0, pinned_bytes = 0;
-};
-
-enum { kModeTable = 0, kModeTokensPinned = 1, kModeTokensDirect = 2 };
-
 struct sqz_gpu_stream {
     int device = 0;
     const uint8_t* data = nullptr;
@@ -1063,131 +1156,13 @@ struct sqz_gpu_stream {
     size_t launched = 0;              // input bytes handed to the device so far
     size_t delivered = 0;             // input bytes whose tokens were returned
     int next_slot = 0, read_slot = 0;
-    int mode = kModeTokensPinned;
+    int kind = kConsumer;             // of its two stages: kTable, kTokens or kConsumer
     bool symbols = false;             // emit symbol words instead of plain tokens
-    Slot slot[2];
+    Stage slot[2];
     const uint64_t* prev_result = nullptr;   // device: previous chunk's result (entry hand-off)
     cudaEvent_t prev_parsed = nullptr;
     cudaEvent_t prev_tabled = nullptr;
 };
-
-// the calling thread's current device is the caller's business: every entry point that has to
-// switch (an explicit stream device, the multi-device call) puts it back on the way out
-struct DeviceScope {
-    int saved = -1;
-    DeviceScope() { if (cudaGetDevice(&saved) != cudaSuccess) { saved = -1; cudaGetLastError(); } }
-    ~DeviceScope() { if (saved >= 0) { cudaSetDevice(saved); } }
-};
-
-static void slot_free(Slot& s) {
-    if (s.stream) { cudaStreamSynchronize(s.stream); }
-    cudaFree(s.d_data); cudaFree(s.d_table); cudaFree(s.d_tokens); cudaFree(s.d_len);
-    cudaFree(s.d_dist); cudaFree(s.d_work); cudaFree(s.d_mwork); cudaFree(s.d_result);
-    cudaFreeHost(s.h_result); cudaFreeHost(s.h_tokens);
-    if (s.done) { cudaEventDestroy(s.done); }
-    if (s.parsed) { cudaEventDestroy(s.parsed); }
-    if (s.tabled) { cudaEventDestroy(s.tabled); }
-    if (s.ahead_of_all) { cudaStreamSynchronize(s.ahead_of_all); cudaStreamDestroy(s.ahead_of_all); }
-    if (s.stream) { cudaStreamDestroy(s.stream); }
-    s = Slot();
-}
-
-static int slot_alloc(Slot& s, int device, size_t chunk, uint32_t max_len, uint32_t max_dist, int mode) {
-    s.device = device; s.cap_chunk = chunk; s.cap_len = max_len; s.cap_dist = max_dist; s.cap_mode = mode;
-    CU(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-    CU(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&s.parsed, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&s.tabled, cudaEventDisableTiming));
-    const size_t data_bytes = (size_t)max_dist + chunk + max_len + 64;
-    CU(cudaMalloc(&s.d_data, data_bytes));
-    CU(cudaMalloc(&s.d_table, chunk * 4));
-    CU(cudaMalloc(&s.d_mwork, sqz_gpu_match_workspace(chunk)));
-    CU(cudaMalloc(&s.d_result, 16));
-    CU(cudaHostAlloc(&s.h_result, 16, cudaHostAllocDefault));
-    s.device_bytes = data_bytes + chunk * 4 + sqz_gpu_match_workspace(chunk);
-    if (mode != kModeTable) {
-        CU(cudaMalloc(&s.d_tokens, chunk * 4 + 16));
-        CU(cudaMalloc(&s.d_work, parse::workspace(chunk)));
-        s.device_bytes += chunk * 4 + parse::workspace(chunk);
-        if (mode == kModeTokensPinned) {
-            CU(cudaHostAlloc(&s.h_tokens, chunk * 4 + 16, cudaHostAllocDefault));
-            s.pinned_bytes = chunk * 4 + 16;
-            int least = 0, greatest = 0;
-            CU(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-            CU(cudaStreamCreateWithPriority(&s.ahead_of_all, cudaStreamNonBlocking, greatest));
-        }
-    } else {
-        CU(cudaMalloc(&s.d_len, chunk * 2));
-        CU(cudaMalloc(&s.d_dist, chunk * 2));
-        s.device_bytes += chunk * 4;
-    }
-    return 0;
-}
-
-// Allocating and freeing gigabytes of device and pinned memory per call costs more than the
-// search of a small input and stalls the device; finished calls park their slots here and the
-// next call with the same shape takes them back.  At most kMaxParked slots and kMaxParkedBytes
-// of device + pinned memory stay parked (oldest out first); sqz_gpu_release() frees them all.
-static std::mutex g_park_mu;
-static std::vector<Slot> g_parked;
-constexpr size_t kMaxParked = 4;
-constexpr size_t kMaxParkedBytes = (size_t)3 << 30;
-
-static int slot_take(Slot& s, int device, size_t chunk, uint32_t max_len, uint32_t max_dist, int mode) {
-    // round the capacity up to a power of two (>= 1 MiB) so that calls of similar size share slots
-    size_t cap = (size_t)1 << 20;
-    while (cap < chunk) { cap <<= 1; }
-    chunk = cap;
-    {
-        std::lock_guard<std::mutex> lk(g_park_mu);
-        for (size_t k = 0; k < g_parked.size(); k++) {
-            const Slot& c = g_parked[k];
-            if (c.device == device && c.cap_mode == mode && c.cap_chunk >= chunk &&
-                c.cap_chunk <= 4 * chunk && c.cap_len >= max_len && c.cap_dist >= max_dist) {
-                s = c;
-                g_parked.erase(g_parked.begin() + (long)k);
-                s.first = 0; s.n = 0; s.busy = false;
-                return 0;
-            }
-        }
-    }
-    int r = slot_alloc(s, device, chunk, max_len, max_dist, mode);
-    if (r != 0) { slot_free(s); }
-    return r;
-}
-
-static void slot_give_back(Slot& s) {
-    if (s.stream == nullptr) { s = Slot(); return; }
-    cudaStreamSynchronize(s.stream);
-    std::vector<Slot> victims;
-    {
-        std::lock_guard<std::mutex> lk(g_park_mu);
-        g_parked.push_back(s);
-        size_t total = 0;
-        for (const Slot& c : g_parked) { total += c.device_bytes + c.pinned_bytes; }
-        while (!g_parked.empty() && (g_parked.size() > kMaxParked || total > kMaxParkedBytes)) {
-            total -= g_parked.front().device_bytes + g_parked.front().pinned_bytes;
-            victims.push_back(g_parked.front());
-            g_parked.erase(g_parked.begin());
-        }
-    }
-    s = Slot();
-    for (Slot& v : victims) { cudaSetDevice(v.device); slot_free(v); }
-}
-
-static void multi_release_all();
-
-extern "C" void sqz_gpu_release(void) {
-    std::vector<Slot> all;
-    {
-        std::lock_guard<std::mutex> lk(g_park_mu);
-        all.swap(g_parked);
-    }
-    DeviceScope keep;
-    for (Slot& c : all) { cudaSetDevice(c.device); slot_free(c); }
-    pool_release_all();
-    multi_release_all();
-}
 
 // device < 0 = the calling thread's current device
 static int ensure_device(int& device) {
@@ -1202,9 +1177,34 @@ static int ensure_device(int& device) {
     return 0;
 }
 
+// the arguments every host-buffer entry point checks, in this order: rules, window, input, device
+// (which ensure_device makes current)
+static int check_call(int& device, uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                      const uint8_t* data, size_t bytes) {
+    if (int r = check_rules(min_len, max_len, max_dist)) { return r; }
+    if (window == 0 || (window & (window - 1)) != 0 || max_dist > window) {
+        return fail(EINVAL, "window must be a power of two and max_dist <= window");
+    }
+    if (data == nullptr && bytes != 0) { return fail(EINVAL, "null input"); }
+    return ensure_device(device);
+}
+
+// Uploads positions [first, first + n) of `data` with their halos and searches them on the stage's
+// stream; the search, not the upload, waits for `after` when there is one.
+static int stage_search(Stage& s, const uint8_t* data, size_t first, size_t n, size_t back, size_t ahead,
+                        uint32_t min_len, uint32_t max_len, uint32_t max_dist, cudaEvent_t after) {
+    s.first = first;
+    s.n = n;
+    s.back = back;
+    CU(cudaMemcpyAsync(s.d_data, data + first - back, back + n + ahead, cudaMemcpyHostToDevice, s.stream));
+    if (after != nullptr) { CU(cudaStreamWaitEvent(s.stream, after, 0)); }
+    return sqz_gpu_match_table_device_ws(s.d_data + back, back, n, ahead, min_len, max_len, max_dist,
+                                         s.d_table, s.d_mwork, s.stream);
+}
+
 // issue everything for the next chunk on its slot; returns without waiting
 static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* dist_out) {
-    Slot& s = st->slot[st->next_slot];
+    Stage& s = st->slot[st->next_slot];
     const size_t first = st->launched;
     size_t n = std::min(st->chunk, st->bytes - first);
     if (st->ramp != 0) {               // short chunks first: the consumer starts after milliseconds
@@ -1213,27 +1213,21 @@ static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* d
     }
     const size_t back = std::min<size_t>(first, st->max_dist);
     const size_t ahead = std::min<size_t>(st->bytes - (first + n), st->max_len);
-    s.first = first;
-    s.n = n;
-    CU(cudaMemcpyAsync(s.d_data, st->data + first - back, back + n + ahead,
-                       cudaMemcpyHostToDevice, s.stream));
-    const uint8_t* d_shard = s.d_data + back;
-    if (st->mode == kModeTokensPinned && st->prev_tabled != nullptr) {
-        // A consumer waits for the chunks in order: two searches sharing the device would both be ready
-        // late.  This chunk's search starts when the one before has its table; only that one's parse and
-        // copy run beside it.
-        CU(cudaStreamWaitEvent(s.stream, st->prev_tabled, 0));
-    }
-    if (int r = sqz_gpu_match_table_device_ws(d_shard, back, n, ahead, st->min_len, st->max_len,
-                                              st->max_dist, s.d_table, s.d_mwork, s.stream)) { return r; }
+    const bool consumer = st->kind == kConsumer;
+    // A consumer waits for the chunks in order: two searches sharing the device would both be ready
+    // late.  This chunk's search starts when the one before has its table; only that one's parse and
+    // copy run beside it.
+    if (int r = stage_search(s, st->data, first, n, back, ahead, st->min_len, st->max_len, st->max_dist,
+                             consumer ? st->prev_tabled : nullptr)) { return r; }
     CU(cudaEventRecord(s.tabled, s.stream));
     st->prev_tabled = s.tabled;
+    const uint8_t* d_shard = s.d_data + back;
     // A consumer's parse and token copy go on a stream of the highest priority: the next chunk's search
     // is queued behind this one's and fills the device as soon as it may -- at equal priority the few
     // small kernels that finish this chunk would wait for free CTA slots until that search is over.
-    cudaStream_t late = st->mode == kModeTokensPinned ? s.ahead_of_all : s.stream;
+    cudaStream_t late = consumer ? s.ahead_of_all : s.stream;
     if (late != s.stream) { CU(cudaStreamWaitEvent(late, s.tabled, 0)); }
-    if (st->mode != kModeTable) {
+    if (st->kind != kTable) {
         const uint32_t* d_entry = nullptr;
         if (st->prev_result != nullptr) {
             CU(cudaStreamWaitEvent(late, st->prev_parsed, 0));
@@ -1245,14 +1239,14 @@ static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* d
         CU(cudaEventRecord(s.parsed, late));
         st->prev_parsed = s.parsed;
         st->prev_result = s.d_result;
-        if (st->mode == kModeTokensPinned) {
+        if (consumer) {
             // the tokens follow right away, exactly as many as there are: the consumer finds them
             // in pinned memory when it asks
             const unsigned grid = (unsigned)std::min<size_t>((n / 4 + 255) / 256 + 1, (size_t)sm_count() * 4);
             tokens_to_host<<<grid, 256, 0, late>>>(s.d_tokens, s.d_result, s.h_tokens);
             LAUNCHED("tokens_to_host");
         }
-        // kModeTokensDirect: the caller copies count x 4 bytes to their final place once it knows the count
+        // kTokens: the caller copies count x 4 bytes to their final place once it knows the count
     } else {
         if (int r = sqz_gpu_unpack_table_device(s.d_table, n, s.d_len, s.d_dist, s.stream)) { return r; }
         CU(cudaMemcpyAsync(len_out + first, s.d_len, n * 2, cudaMemcpyDeviceToHost, s.stream));
@@ -1278,34 +1272,37 @@ static size_t default_chunk(size_t bytes, bool consumer) {
 
 static int stream_open(sqz_gpu_stream** out, int device, const uint8_t* data, size_t bytes,
                        uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
-                       size_t chunk, int mode, bool short_start = false) {
+                       size_t chunk, int kind, bool short_start = false) {
     *out = nullptr;
-    if (int r = check_rules(min_len, max_len, max_dist)) { return r; }
-    if (window == 0 || (window & (window - 1)) != 0 || max_dist > window) {
-        return fail(EINVAL, "window must be a power of two and max_dist <= window");
-    }
-    if (data == nullptr && bytes != 0) { return fail(EINVAL, "null input"); }
-    if (int r = ensure_device(device)) { return r; }
+    if (int r = check_call(device, window, min_len, max_len, max_dist, data, bytes)) { return r; }
     sqz_gpu_stream* st = new (std::nothrow) sqz_gpu_stream();
     if (st == nullptr) { return fail(ENOMEM, "out of host memory"); }
     st->device = device;
     st->data = data;
     st->bytes = bytes;
     st->min_len = min_len; st->max_len = max_len; st->max_dist = max_dist;
-    st->chunk = chunk ? chunk : default_chunk(bytes, mode == kModeTokensPinned);
-    st->mode = mode;
+    st->chunk = chunk ? chunk : default_chunk(bytes, kind == kConsumer);
+    st->kind = kind;
     // token streams with the default chunking start with short chunks: 2, 4, 8, 16 MiB, then 32 MiB
-    if (mode == kModeTokensPinned && chunk == 0 && st->chunk > ((size_t)2 << 20)) { st->ramp = (size_t)2 << 20; }
+    if (kind == kConsumer && chunk == 0 && st->chunk > ((size_t)2 << 20)) { st->ramp = (size_t)2 << 20; }
     if (short_start && chunk >= ((size_t)4 << 20)) { st->ramp = chunk / 4; }
     const int slots = bytes > (st->ramp ? st->ramp : st->chunk) ? 2 : 1;
     for (int k = 0; k < slots && bytes > 0; k++) {
-        if (int r = slot_take(st->slot[k], device, st->chunk, max_len, max_dist, mode)) {
+        if (int r = stage_take(st->slot[k], device, kind, st->chunk)) {
             sqz_gpu_stream_close(st);
             return r;
         }
     }
     *out = st;
     return 0;
+}
+
+// Waits for both slots, parks them and deletes the stream; returns rc, or the first error of the
+// waits when rc is 0.
+static int stream_finish(sqz_gpu_stream* st, int rc) {
+    for (Stage& s : st->slot) { rc = stage_finish(s, rc); }
+    delete st;
+    return rc;
 }
 
 extern "C" int sqz_gpu_stream_open(sqz_gpu_stream** st, int device, const uint8_t* data,
@@ -1321,7 +1318,7 @@ extern "C" int sqz_gpu_stream_open(sqz_gpu_stream** st, int device, const uint8_
     }
     DeviceScope keep;
     if (int r = stream_open(st, device, data, bytes, window, min_len, max_len, max_dist,
-                            chunk_bytes, kModeTokensPinned, (flags & SQZ_GPU_STREAM_SHORT_START) != 0)) { return r; }
+                            chunk_bytes, kConsumer, (flags & SQZ_GPU_STREAM_SHORT_START) != 0)) { return r; }
     (*st)->symbols = (flags & SQZ_GPU_STREAM_SYMBOLS) != 0;
     if (bytes > 0) {
         if (int r = stream_launch_next(*st, nullptr, nullptr)) {
@@ -1347,7 +1344,7 @@ extern "C" int sqz_gpu_stream_next(sqz_gpu_stream* st, const uint32_t** tokens, 
         if (int r = stream_launch_next(st, nullptr, nullptr)) { return r; }
     }
     const auto t1 = std::chrono::steady_clock::now();
-    Slot& s = st->slot[st->read_slot];
+    Stage& s = st->slot[st->read_slot];
     CU(cudaEventSynchronize(s.done));
     if (trace) {
         const auto t2 = std::chrono::steady_clock::now();
@@ -1369,9 +1366,7 @@ extern "C" void sqz_gpu_stream_close(sqz_gpu_stream* st) {
     if (st == nullptr) { return; }
     DeviceScope keep;
     cudaSetDevice(st->device);
-    slot_give_back(st->slot[0]);
-    slot_give_back(st->slot[1]);
-    delete st;
+    stream_finish(st, 0);
 }
 
 // One-shot token call: the chunks' tokens go straight from device memory to their final place in
@@ -1385,17 +1380,17 @@ extern "C" int sqz_gpu_tokens(const uint8_t* data, size_t bytes, uint32_t window
     *n_tokens = 0;
     sqz_gpu_stream* st = nullptr;
     DeviceScope keep;
-    if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kModeTokensDirect)) {
+    if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kTokens)) {
         return r;
     }
     size_t total = 0;
     int rc = 0;
     if (bytes > 0) { rc = stream_launch_next(st, nullptr, nullptr); }
     while (rc == 0 && st->delivered < st->bytes) {
-        Slot& s = st->slot[st->read_slot];
+        Stage& s = st->slot[st->read_slot];
         // the other slot is free (its copy was queued before its `done`): keep the device busy
         if (st->launched < st->bytes) {
-            Slot& o = st->slot[st->next_slot];
+            Stage& o = st->slot[st->next_slot];
             if (o.busy) {
                 cudaError_t ce = cudaEventSynchronize(o.done);
                 if (ce != cudaSuccess) { rc = fail(cuda_code(ce), "cudaEventSynchronize", ce); break; }
@@ -1419,13 +1414,7 @@ extern "C" int sqz_gpu_tokens(const uint8_t* data, size_t bytes, uint32_t window
         st->delivered = s.first + s.n;
         st->read_slot ^= 1;
     }
-    for (int k = 0; k < 2; k++) {
-        if (st->slot[k].stream != nullptr) {
-            cudaError_t ce = cudaStreamSynchronize(st->slot[k].stream);
-            if (ce != cudaSuccess && rc == 0) { rc = fail(cuda_code(ce), "cudaStreamSynchronize", ce); }
-        }
-    }
-    sqz_gpu_stream_close(st);
+    rc = stream_finish(st, rc);
     *n_tokens = total;
     if (rc == 0 && total > tokens_cap) { rc = fail(E2BIG, "token buffer too small"); }
     return rc;
@@ -1439,12 +1428,12 @@ extern "C" int sqz_gpu_match_table(const uint8_t* data, size_t bytes, uint32_t w
     }
     sqz_gpu_stream* st = nullptr;
     DeviceScope keep;
-    if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kModeTable)) {
+    if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kTable)) {
         return r;
     }
     int rc = 0;
     while (rc == 0 && st->launched < st->bytes) {
-        Slot& s = st->slot[st->next_slot];
+        Stage& s = st->slot[st->next_slot];
         if (s.busy) {                      // reuse only after its copies have landed
             cudaError_t ce = cudaEventSynchronize(s.done);
             if (ce != cudaSuccess) { rc = fail(cuda_code(ce), "cudaEventSynchronize", ce); break; }
@@ -1452,14 +1441,7 @@ extern "C" int sqz_gpu_match_table(const uint8_t* data, size_t bytes, uint32_t w
         }
         rc = stream_launch_next(st, len_out, dist_out);
     }
-    for (int k = 0; k < 2; k++) {
-        if (st->slot[k].stream != nullptr) {
-            cudaError_t ce = cudaStreamSynchronize(st->slot[k].stream);
-            if (ce != cudaSuccess && rc == 0) { rc = fail(cuda_code(ce), "cudaStreamSynchronize", ce); }
-        }
-    }
-    sqz_gpu_stream_close(st);
-    return rc;
+    return stream_finish(st, rc);
 }
 
 // ---------------------------------------------------------------------------
@@ -1473,127 +1455,38 @@ extern "C" int sqz_gpu_match_table(const uint8_t* data, size_t bytes, uint32_t w
 // their counts: device -> host when tokens_out is host memory, peer-to-peer (cudaMemcpyPeerAsync
 // over NVLink) when it is device memory.
 // ---------------------------------------------------------------------------
-struct MultiPart {
-    int device = 0;
-    size_t first = 0, n = 0, back = 0, ahead = 0;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t mapped = nullptr, parsed = nullptr;
-    uint8_t* d_data = nullptr;
-    uint32_t* d_table = nullptr;
-    uint32_t* d_tokens = nullptr;
-    void* d_work = nullptr;
-    void* d_mwork = nullptr;
-    uint16_t* d_map = nullptr;
-    uint64_t* d_result = nullptr;
-    uint16_t* h_map = nullptr;        // pinned: exit map
-    uint64_t* h_result = nullptr;     // pinned: count, overshoot
-    size_t cap_n = 0, cap_data = 0;   // what the buffers hold (parts are recycled between calls)
-};
-
-static void multi_free(MultiPart& p) {
-    cudaSetDevice(p.device);
-    if (p.stream) { cudaStreamSynchronize(p.stream); }
-    cudaFree(p.d_data); cudaFree(p.d_table); cudaFree(p.d_tokens); cudaFree(p.d_work);
-    cudaFree(p.d_mwork); cudaFree(p.d_map); cudaFree(p.d_result);
-    cudaFreeHost(p.h_map); cudaFreeHost(p.h_result);
-    if (p.mapped) { cudaEventDestroy(p.mapped); }
-    if (p.parsed) { cudaEventDestroy(p.parsed); }
-    if (p.stream) { cudaStreamDestroy(p.stream); }
-    p = MultiPart();
-}
-
-// Like the slots of the single-device pipeline, the per-device buffers of a multi-device call are
-// kept for the next call of a similar size (allocating ten gigabytes takes longer than searching a
-// small input); at most kMultiParked of them, and only parts below kMultiParkBytes of device memory.
-static std::vector<MultiPart> g_multi_parked;      // guarded by g_park_mu
-constexpr size_t kMultiParked = 8;
-constexpr size_t kMultiParkBytes = (size_t)12 << 30;
-
-static size_t multi_bytes(const MultiPart& p) { return p.cap_data + p.cap_n * 8 + parse::workspace(p.cap_n) + sqz_gpu_match_workspace(p.cap_n); }
-
-static int multi_alloc(MultiPart& p) {
-    const size_t need_data = p.back + p.n + p.ahead + 64;
-    {
-        std::lock_guard<std::mutex> lk(g_park_mu);
-        for (size_t k = 0; k < g_multi_parked.size(); k++) {
-            const MultiPart& c = g_multi_parked[k];
-            if (c.device == p.device && c.cap_n >= p.n && c.cap_n <= 2 * p.n + ((size_t)1 << 20) && c.cap_data >= need_data) {
-                MultiPart t = c;
-                g_multi_parked.erase(g_multi_parked.begin() + (long)k);
-                t.first = p.first; t.n = p.n; t.back = p.back; t.ahead = p.ahead;
-                p = t;
-                CU(cudaSetDevice(p.device));
-                return 0;
-            }
-        }
-    }
-    CU(cudaSetDevice(p.device));
-    p.cap_n = (std::max<size_t>(p.n, 1) + ((size_t)1 << 20) - 1) >> 20 << 20;
-    p.cap_data = p.cap_n + (size_t)sqz_gpu_max_dist_limit + sqz_gpu_max_len_limit + 64;
-    CU(cudaStreamCreateWithFlags(&p.stream, cudaStreamNonBlocking));
-    CU(cudaEventCreateWithFlags(&p.mapped, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&p.parsed, cudaEventDisableTiming));
-    CU(cudaMalloc(&p.d_data, p.cap_data));
-    CU(cudaMalloc(&p.d_table, p.cap_n * 4));
-    CU(cudaMalloc(&p.d_tokens, p.cap_n * 4 + 16));
-    CU(cudaMalloc(&p.d_work, parse::workspace(p.cap_n)));
-    CU(cudaMalloc(&p.d_mwork, sqz_gpu_match_workspace(p.cap_n)));
-    CU(cudaMalloc(&p.d_map, parse::kMapStride * 2));
-    CU(cudaMalloc(&p.d_result, 16));
-    CU(cudaHostAlloc(&p.h_map, parse::kMapStride * 2, cudaHostAllocDefault));
-    CU(cudaHostAlloc(&p.h_result, 16, cudaHostAllocDefault));
-    return 0;
-}
-
-static void multi_give_back(MultiPart& p) {
-    if (p.stream == nullptr || p.cap_n == 0 || multi_bytes(p) > kMultiParkBytes) { multi_free(p); return; }
-    cudaSetDevice(p.device);
-    cudaStreamSynchronize(p.stream);
-    MultiPart victim;
-    {
-        std::lock_guard<std::mutex> lk(g_park_mu);
-        g_multi_parked.push_back(p);
-        if (g_multi_parked.size() > kMultiParked) { victim = g_multi_parked.front(); g_multi_parked.erase(g_multi_parked.begin()); }
-    }
-    p = MultiPart();
-    if (victim.stream != nullptr) { multi_free(victim); }
-}
-
-static void multi_release_all() {
-    std::vector<MultiPart> all;
-    {
-        std::lock_guard<std::mutex> lk(g_park_mu);
-        all.swap(g_multi_parked);
-    }
-    for (MultiPart& p : all) { multi_free(p); }
-}
-
-static int multi_run(std::vector<MultiPart>& parts, const uint8_t* data, uint32_t min_len, uint32_t max_len,
-                     uint32_t max_dist, uint32_t* tokens_out, size_t tokens_cap, bool out_on_device,
-                     int out_device, size_t* n_tokens, size_t* shard_tokens) {
+static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_t* data, size_t bytes,
+                     uint32_t min_len, uint32_t max_len, uint32_t max_dist, uint32_t* tokens_out,
+                     size_t tokens_cap, bool out_on_device, int out_device, size_t* n_tokens,
+                     size_t* shard_tokens) {
     // phase A on every device at once: upload, match table, composed exit map
-    for (MultiPart& p : parts) {
-        if (p.n == 0) { continue; }
-        if (int r = multi_alloc(p)) { return r; }
-        CU(cudaMemcpyAsync(p.d_data, data + p.first - p.back, p.back + p.n + p.ahead, cudaMemcpyHostToDevice, p.stream));
-        const uint8_t* d_shard = p.d_data + p.back;
-        if (int r = sqz_gpu_match_table_device_ws(d_shard, p.back, p.n, p.ahead, min_len, max_len, max_dist,
-                                                  p.d_table, p.d_mwork, p.stream)) { return r; }
-        if (int r = sqz_gpu_parse_exit_map_device(p.d_table, p.n, min_len, max_len, p.d_work, p.d_map, p.stream)) { return r; }
-        CU(cudaMemcpyAsync(p.h_map, p.d_map, (size_t)max_len * 2, cudaMemcpyDeviceToHost, p.stream));
-        CU(cudaEventRecord(p.mapped, p.stream));
+    const size_t base = bytes / parts.size(), extra = bytes % parts.size();
+    size_t first = 0;
+    for (size_t g = 0; g < parts.size(); g++) {
+        const size_t n = base + (g < extra ? 1 : 0);
+        if (n > 0) {
+            Stage& p = parts[g];
+            CU(cudaSetDevice(devices[g]));
+            if (int r = stage_take(p, devices[g], kTokens, n)) { return r; }
+            if (int r = stage_search(p, data, first, n, std::min<size_t>(first, max_dist),
+                                     std::min<size_t>(bytes - (first + n), max_len), min_len, max_len, max_dist,
+                                     nullptr)) { return r; }
+            if (int r = sqz_gpu_parse_exit_map_device(p.d_table, n, min_len, max_len, p.d_work, p.d_map, p.stream)) { return r; }
+            CU(cudaMemcpyAsync(p.h_map, p.d_map, (size_t)max_len * 2, cudaMemcpyDeviceToHost, p.stream));
+            CU(cudaEventRecord(p.tabled, p.stream));
+        }
+        first += n;
     }
     // seams: shard g+1 is entered where shard g's last token ends
     uint32_t entry = 0;
-    for (MultiPart& p : parts) {
+    for (Stage& p : parts) {
         if (p.n == 0) { continue; }
         CU(cudaSetDevice(p.device));
-        CU(cudaEventSynchronize(p.mapped));
-        const uint8_t* d_shard = p.d_data + p.back;
+        CU(cudaEventSynchronize(p.tabled));
         if (entry >= max_len) { return fail(EIO, "seam entry out of range"); }
         const uint32_t next_entry = p.h_map[entry];
-        if (int r = parse_launch(d_shard, p.d_table, p.n, nullptr, entry, min_len, max_len, p.d_tokens, p.n,
-                                 p.d_work, p.d_result, p.stream)) { return r; }
+        if (int r = parse_launch(p.d_data + p.back, p.d_table, p.n, nullptr, entry, min_len, max_len, p.d_tokens,
+                                 p.n, p.d_work, p.d_result, p.stream)) { return r; }
         CU(cudaMemcpyAsync(p.h_result, p.d_result, 16, cudaMemcpyDeviceToHost, p.stream));
         CU(cudaEventRecord(p.parsed, p.stream));
         entry = next_entry;
@@ -1601,7 +1494,7 @@ static int multi_run(std::vector<MultiPart>& parts, const uint8_t* data, uint32_
     // concatenation in shard order, every copy sized by its shard's count
     size_t total = 0;
     for (size_t g = 0; g < parts.size(); g++) {
-        MultiPart& p = parts[g];
+        Stage& p = parts[g];
         size_t c = 0;
         if (p.n != 0) {
             CU(cudaSetDevice(p.device));
@@ -1620,11 +1513,6 @@ static int multi_run(std::vector<MultiPart>& parts, const uint8_t* data, uint32_
         if (shard_tokens != nullptr) { shard_tokens[g] = c; }
         total += c;
     }
-    for (MultiPart& p : parts) {
-        if (p.n == 0) { continue; }
-        CU(cudaSetDevice(p.device));
-        CU(cudaStreamSynchronize(p.stream));
-    }
     *n_tokens = total;
     if (entry != 0) { return fail(EIO, "the parse does not end at the end of the input"); }
     return total > tokens_cap ? fail(E2BIG, "token buffer too small") : 0;
@@ -1637,21 +1525,14 @@ extern "C" int sqz_gpu_tokens_multi(const int* devices, int n_devices, const uin
     if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
     *n_tokens = 0;
     if (devices == nullptr || n_devices < 1 || n_devices > kMaxDevices) { return fail(EINVAL, "bad device list"); }
-    if (int r = check_rules(min_len, max_len, max_dist)) { return r; }
-    if (window == 0 || (window & (window - 1)) != 0 || max_dist > window) {
-        return fail(EINVAL, "window must be a power of two and max_dist <= window");
-    }
-    if (data == nullptr && bytes != 0) { return fail(EINVAL, "null input"); }
-    int count = 0;
-    cudaError_t ce = cudaGetDeviceCount(&count);
-    if (ce != cudaSuccess || count == 0) {
-        return fail(ENODEV, "no CUDA device: the match search has no CPU fallback", ce);
-    }
+    DeviceScope keep;
+    int device = devices[0];
+    if (int r = check_call(device, window, min_len, max_len, max_dist, data, bytes)) { return r; }
+    const int count = sqz_gpu_device_count();
     for (int g = 0; g < n_devices; g++) {
         // (a device may be listed more than once: its shards then share it, each on its own stream)
         if (devices[g] < 0 || devices[g] >= count) { return fail(ENODEV, "no such CUDA device"); }
     }
-    DeviceScope keep;
     // where do the tokens go: host memory, or device memory (then peer copies gather them there)
     bool out_on_device = false;
     int out_device = devices[0];
@@ -1670,30 +1551,16 @@ extern "C" int sqz_gpu_tokens_multi(const int* devices, int n_devices, const uin
             CU(cudaDeviceCanAccessPeer(&can, devices[g], out_device));
             if (can) {
                 CU(cudaSetDevice(devices[g]));
-                ce = cudaDeviceEnablePeerAccess(out_device, 0);
+                cudaError_t ce = cudaDeviceEnablePeerAccess(out_device, 0);
                 if (ce != cudaSuccess && ce != cudaErrorPeerAccessAlreadyEnabled) { return fail(cuda_code(ce), "cudaDeviceEnablePeerAccess", ce); }
                 cudaGetLastError();
             }   // without peer access cudaMemcpyPeerAsync still works, staged through the host
         }
     }
-    std::vector<MultiPart> parts((size_t)n_devices);
-    const size_t base = bytes / (size_t)n_devices, extra = bytes % (size_t)n_devices;
-    size_t first = 0;
-    for (int g = 0; g < n_devices; g++) {
-        MultiPart& p = parts[(size_t)g];
-        p.device = devices[g];
-        p.first = first;
-        p.n = base + ((size_t)g < extra ? 1 : 0);
-        p.back = std::min<size_t>(first, max_dist);
-        p.ahead = std::min<size_t>(bytes - (first + p.n), max_len);
-        first += p.n;
-    }
-    const int rc = multi_run(parts, data, min_len, max_len, max_dist, tokens_out, tokens_cap, out_on_device,
-                             out_device, n_tokens, shard_tokens);
-    for (MultiPart& p : parts) {
-        if (rc == 0 && p.stream != nullptr) { multi_give_back(p); }
-        else if (p.stream != nullptr || p.d_data != nullptr) { multi_free(p); }
-    }
+    std::vector<Stage> parts((size_t)n_devices);
+    int rc = multi_run(parts, devices, data, bytes, min_len, max_len, max_dist, tokens_out, tokens_cap,
+                       out_on_device, out_device, n_tokens, shard_tokens);
+    for (Stage& p : parts) { rc = stage_finish(p, rc); }
     return rc;
 }
 
