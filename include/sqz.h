@@ -105,7 +105,10 @@ struct sqz {
                                            threads working on segments + the caller's thread appending them in
                                            order; 0 = automatic (1 below 64 Ki tokens, 2 below 1 Mi tokens or on
                                            fewer than 8 cores, else 4); same bytes in every case (sqz_codec.c) */
-    int32_t  reserved;
+    int32_t  lazy;                      /* sqz_compress's parse: 0 (sqz_init) = greedy, the reference's exact
+                                           stream; 1 = lazy matching (SQZ_GPU_STREAM_LAZY in sqz_gpu.h): about
+                                           2 % smaller on text and code, slightly larger on data that does not
+                                           compress, read by every decoder; other values: EINVAL */
     struct sqz_tree lit;
     uint8_t len_index[sqz_max_len + 2]; /* len -> length bucket, squeeze.h:151-161.  Also keeps the two tree
                                            headers on different cache lines: with two coder threads each
@@ -128,7 +131,8 @@ void sqz_read_header(struct sqz_bitstream* bs, uint64_t* bytes, uint8_t* win_bit
 void sqz_init(struct sqz* s);
 
 /* LZ77 (GPU) + adaptive Huffman (host).  window must be a power of two in
- * [2^10, 2^15].  Errors are reported in s->error.                            */
+ * [2^10, 2^15].  The parse is greedy unless s->lazy is 1.  Errors are
+ * reported in s->error.                                                      */
 void sqz_compress(struct sqz* s, struct sqz_bitstream* bs,
                   const uint8_t* data, uint64_t bytes, uint32_t window);
 

@@ -110,10 +110,19 @@ int sqz_gpu_tokens_multi(const int* devices, int n_devices,
  * first two are a quarter and a half of it.  The searches of consecutive
  * chunks run one after the other (a consumer wants them in order, not both
  * late), a chunk's parse and copy at the highest stream priority beside the
- * next chunk's search.                                                      */
+ * next chunk's search.
+ * SQZ_GPU_STREAM_LAZY parses with lazy matching instead of the greedy rule:
+ * at a position whose match reaches min_len, the literal is emitted instead
+ * when the next position has a strictly longer match, and the decision is
+ * taken again there (len at the end of the input counts as 0).  About 2 %
+ * smaller streams of text and code, slightly larger ones of data that does
+ * not compress; any decoder reads them.  Only this entry point has the lazy
+ * parse: sqz_gpu_tokens, sqz_gpu_tokens_multi and the device-buffer parse
+ * entry points below are greedy.                                            */
 typedef struct sqz_gpu_stream sqz_gpu_stream;
 #define SQZ_GPU_STREAM_SYMBOLS 1u       /* deliver symbol words instead of plain tokens */
 #define SQZ_GPU_STREAM_SHORT_START 2u   /* explicit chunk_bytes: start with chunk_bytes / 4, then / 2 */
+#define SQZ_GPU_STREAM_LAZY 8u          /* lazy matching instead of the greedy parse (combines with the others) */
 int  sqz_gpu_stream_open(sqz_gpu_stream** st, int device,
                          const uint8_t* data, size_t bytes,
                          uint32_t window, uint32_t min_len, uint32_t max_len,

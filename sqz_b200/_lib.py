@@ -54,7 +54,7 @@ class State(C.Structure):
         ("error", C.c_int32), ("device", C.c_int32), ("bs", C.POINTER(Bitstream)),
         ("tokens", C.c_uint64), ("matches", C.c_uint64),
         ("search_seconds", C.c_double), ("entropy_seconds", C.c_double),
-        ("coder_threads", C.c_int32), ("reserved", C.c_int32),
+        ("coder_threads", C.c_int32), ("lazy", C.c_int32),
         ("lit", Tree), ("len_index", C.c_uint8 * 259), ("apart", C.c_uint8 * 64), ("pos", Tree),
         ("lit_store", _store(512)), ("pos_store", _store(32)),
         ("lit_lut", C.c_uint16 * 1024), ("pos_lut", C.c_uint16 * 64),

@@ -123,10 +123,12 @@ def _capacity(nbytes: int) -> int:
 
 
 def compress(data, win_bits: int = 15, file_mode: bool = False, stats: dict | None = None,
-             threads: int = 0, into=None):
+             threads: int = 0, into=None, lazy: bool = False):
     """squeeze.write_header + squeeze.compress: GPU search, host entropy stage.  Returns the bitstream as
     bytes -- or, with `into` (a C-contiguous writable uint8 array of at least capacity(len(data)) bytes, the
-    caller's buffer as in the C API), a view of the part of it that was written, without a copy."""
+    caller's buffer as in the C API), a view of the part of it that was written, without a copy.
+    lazy=True parses with lazy matching (struct sqz's `lazy`): a smaller stream on text and code, in the
+    same format; the default greedy parse gives the reference's exact bytes."""
     L = _lib.load()
     d = _u8(data)
     if into is not None:
@@ -155,6 +157,7 @@ def compress(data, win_bits: int = 15, file_mode: bool = False, stats: dict | No
     s = State()
     L.sqz_init(C.byref(s))
     s.coder_threads = threads
+    s.lazy = 1 if lazy else 0
     L.sqz_compress(C.byref(s), C.byref(bs), d.ctypes.data_as(u8p), d.size, 1 << win_bits)
     _check(s.error, "sqz_compress")
     if stats is not None:

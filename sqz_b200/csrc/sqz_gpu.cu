@@ -7,7 +7,8 @@
 // Results are bit-exact: for every position the longest common prefix with a
 // candidate at distance 1..max_dist (capped by max_len and the end of data),
 // the nearest candidate among equals; then the orbit of position 0 under
-// next[i] = i + (len[i] >= min_len ? len[i] : 1) as the token stream.
+// next[i] = i + (len[i] >= min_len ? len[i] : 1) as the token stream.  The streaming
+// pipeline can parse with lazy matching instead (SQZ_GPU_STREAM_LAZY, namespace parse).
 //
 // There is no CPU fallback in this file: without a device every entry point
 // returns ENODEV.
@@ -213,6 +214,8 @@ __global__ void unpack_table(const uint32_t* __restrict__ table, size_t n,
 //   parse_walk<0>    per block (one warp, steps staged in shared memory): number of tokens on the real path
 //   scan_counts      exclusive prefix sum -> output offsets, total
 //   parse_walk<1>    per block: the same walk, then all lanes write the tokens (or symbol words)
+// The lazy parse (kLazy) is the same machinery with another step, which also reads table[i + 1]: its
+// steps are still 1 or len <= max_len, so entries, overshoots and maps keep their bounds.
 // ---------------------------------------------------------------------------
 namespace parse {
 
@@ -274,12 +277,28 @@ static Work carve(void* d_work, size_t n) {
     return w;
 }
 
-__device__ __forceinline__ uint32_t step_of(uint32_t word, uint32_t min_len) {
-    const uint32_t len = word >> 16;
-    return len >= min_len ? len : 1u;
+// The decision at a parse position i, from its table word and, for the lazy parse, table[i + 1] (at
+// the shard's last position table[n], which the caller provides).  Greedy: the match when it reaches
+// min_len.  Lazy: not when the next position has a strictly longer one -- then the literal, and the
+// decision is taken again at i + 1.  Either way the step is 1 or len <= max_len, which is all the
+// exit maps and the walk rely on.
+template <bool kLazy>
+__device__ __forceinline__ uint32_t next_word(const uint32_t* __restrict__ table, size_t i) {
+    return kLazy ? table[i + 1] : 0u;
 }
 
-template <int kPB>
+template <bool kLazy>
+__device__ __forceinline__ bool takes_match(uint32_t word, uint32_t next, uint32_t min_len) {
+    const uint32_t len = word >> 16;
+    return len >= min_len && !(kLazy && (next >> 16) > len);
+}
+
+template <bool kLazy>
+__device__ __forceinline__ uint32_t step_of(uint32_t word, uint32_t next, uint32_t min_len) {
+    return takes_match<kLazy>(word, next, min_len) ? word >> 16 : 1u;
+}
+
+template <int kPB, bool kLazy>
 __global__ void __launch_bounds__(256)
 parse_exit_map(const uint32_t* __restrict__ table, size_t n, uint32_t min_len,
                uint32_t max_len, uint16_t* __restrict__ exit_map) {
@@ -287,7 +306,7 @@ parse_exit_map(const uint32_t* __restrict__ table, size_t n, uint32_t min_len,
     const size_t b0 = (size_t)blockIdx.x * kPB;
     const int size = (int)min((size_t)kPB, n - b0);            // positions in this block
     for (int p = threadIdx.x; p < size; p += blockDim.x) {
-        jump[p] = (uint16_t)(p + step_of(table[b0 + p], min_len));
+        jump[p] = (uint16_t)(p + step_of<kLazy>(table[b0 + p], next_word<kLazy>(table, b0 + p), min_len));
     }
     __syncthreads();
     // asynchronous pointer doubling: every value stored is a point on p's own
@@ -430,9 +449,11 @@ __device__ __forceinline__ uint32_t symbols_of_match(uint32_t len, uint32_t dist
 // notes the positions it visits; then all lanes turn those positions into tokens (table word
 // or literal byte, optionally as the coder's symbol word) and store them side by side.
 // kEmit = false: count only (first pass, feeds the scan that places every block's tokens).
+// The emit pass takes the same decision as the step (takes_match): under the lazy rule a literal
+// can sit where the table word is a match.
 constexpr int kParseWarps = 2;
 
-template <bool kEmit, bool kSymbols, int kPB>
+template <bool kEmit, bool kSymbols, int kPB, bool kLazy>
 __global__ void __launch_bounds__(32 * kParseWarps)
 parse_walk(const uint8_t* __restrict__ shard, const uint32_t* __restrict__ table, size_t n,
            size_t blocks, uint32_t min_len, const uint32_t* __restrict__ block_entry,
@@ -446,7 +467,7 @@ parse_walk(const uint8_t* __restrict__ shard, const uint32_t* __restrict__ table
     const size_t b0 = b * kPB;
     const uint32_t size = (uint32_t)min((size_t)kPB, n - b0);
     for (uint32_t p = lane; p < size; p += 32) {
-        step_s[warp][p] = (uint16_t)step_of(table[b0 + p], min_len);
+        step_s[warp][p] = (uint16_t)step_of<kLazy>(table[b0 + p], next_word<kLazy>(table, b0 + p), min_len);
     }
     __syncwarp();
     uint32_t c = 0;
@@ -470,8 +491,11 @@ parse_walk(const uint8_t* __restrict__ shard, const uint32_t* __restrict__ table
         const uint32_t w = table[b0 + p];
         const uint32_t len = w >> 16;
         uint32_t t;
-        if (len >= min_len) { t = kSymbols ? symbols_of_match(len, w & 0xFFFF) : w; }
-        else                { t = shard[b0 + p]; }
+        if (takes_match<kLazy>(w, next_word<kLazy>(table, b0 + p), min_len)) {
+            t = kSymbols ? symbols_of_match(len, w & 0xFFFF) : w;
+        } else {
+            t = shard[b0 + p];
+        }
         if (first + j < cap) { tokens[first + j] = t; }
     }
 }
@@ -732,7 +756,7 @@ static int stage_alloc(Stage& s) {
     CU(cudaEventCreateWithFlags(&s.parsed, cudaEventDisableTiming));
     CU(cudaEventCreateWithFlags(&s.tabled, cudaEventDisableTiming));
     CU(dev(&s.d_data, (size_t)sqz_gpu_max_dist_limit + s.cap + sqz_gpu_max_len_limit + 64));
-    CU(dev(&s.d_table, s.cap * 4));
+    CU(dev(&s.d_table, s.cap * 4 + 4));   // + the seam word a lazy parse reads after a full shard
     CU(dev(&s.d_result, 16));
     CU(pin(&s.h_result, 16));
     if (s.kind == kTable) {
@@ -1024,24 +1048,47 @@ extern "C" int sqz_gpu_unpack_table_device(const uint32_t* d_table, size_t n,
 
 extern "C" size_t sqz_gpu_parse_workspace(size_t n) { return parse::workspace(n); }
 
+// lazy: the lazy rule, which reads d_table[n] as well
 static int parse_maps(const uint32_t* d_table, size_t n, uint32_t min_len, uint32_t max_len,
-                      const parse::Work& w, cudaStream_t s) {
-    if (w.pb == parse::kPBSmall) {
-        parse::parse_exit_map<parse::kPBSmall><<<(unsigned)w.blocks, 256, 0, s>>>(d_table, n, min_len, max_len, w.exit_map);
-    } else {
-        parse::parse_exit_map<parse::kPBLarge><<<(unsigned)w.blocks, 256, 0, s>>>(d_table, n, min_len, max_len, w.exit_map);
-    }
+                      const parse::Work& w, cudaStream_t s, bool lazy) {
+#define SQZ_MAP(PB, LAZY) parse::parse_exit_map<PB, LAZY><<<(unsigned)w.blocks, 256, 0, s>>>(d_table, n, min_len, max_len, \
+                                                                                             w.exit_map)
+    if (lazy) { if (w.pb == parse::kPBSmall) { SQZ_MAP(parse::kPBSmall, true); } else { SQZ_MAP(parse::kPBLarge, true); } }
+    else      { if (w.pb == parse::kPBSmall) { SQZ_MAP(parse::kPBSmall, false); } else { SQZ_MAP(parse::kPBLarge, false); } }
+#undef SQZ_MAP
     LAUNCHED("parse_exit_map");
     parse::chain_groups<<<(unsigned)w.groups, 256, 0, s>>>(w.exit_map, w.blocks, w.group, max_len, w.group_map);
     LAUNCHED("chain_groups");
     return 0;
 }
 
-// entry either from device memory (d_entry != null) or immediate
+// the two walks of the parse (count, then emit) with the scan that places every block's tokens between them
+template <int kPB, bool kLazy>
+static int parse_walks(const uint8_t* d_shard, const uint32_t* d_table, size_t n, uint32_t min_len,
+                       const parse::Work& w, uint32_t* d_tokens, size_t cap, uint64_t* d_result,
+                       cudaStream_t s, bool symbols) {
+    const unsigned wb = (unsigned)((w.blocks + parse::kParseWarps - 1) / parse::kParseWarps);
+    const unsigned wt = 32 * parse::kParseWarps;
+    parse::parse_walk<false, false, kPB, kLazy><<<wb, wt, 0, s>>>(d_shard, d_table, n, w.blocks, min_len, w.block_entry,
+                                                                  w.count, nullptr, nullptr, 0);
+    LAUNCHED("parse_count");
+    parse::scan_counts<<<1, 1024, 0, s>>>(w.count, w.blocks, w.offset, d_result);
+    LAUNCHED("scan_counts");
+#define SQZ_EMIT(SYM) parse::parse_walk<true, SYM, kPB, kLazy><<<wb, wt, 0, s>>>(d_shard, d_table, n, w.blocks, min_len, \
+                                                                                 w.block_entry, nullptr, w.offset, d_tokens, cap)
+    if (symbols) { SQZ_EMIT(true); } else { SQZ_EMIT(false); }
+#undef SQZ_EMIT
+    LAUNCHED("parse_emit");
+    return 0;
+}
+
+// entry either from device memory (d_entry != null) or immediate; lazy: the lazy rule, for which
+// d_table holds n + 1 words (the last one the best match at the first position after the shard, 0
+// at the end of the input)
 static int parse_launch(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
                         const uint32_t* d_entry, uint32_t entry, uint32_t min_len,
                         uint32_t max_len, uint32_t* d_tokens, size_t cap, void* d_work,
-                        uint64_t* d_result, cudaStream_t s, bool symbols = false) {
+                        uint64_t* d_result, cudaStream_t s, bool symbols = false, bool lazy = false) {
     if (n == 0) {
         // nothing to parse: count 0, overshoot = entry
         CU(cudaMemsetAsync(d_result, 0, 16, s));
@@ -1054,32 +1101,19 @@ static int parse_launch(const uint8_t* d_shard, const uint32_t* d_table, size_t 
     }
     parse::Work w = parse::carve(d_work, n);
     if (w.blocks > 0x7FFFFFFFull) { return fail(EINVAL, "shard too large for one launch"); }
-    if (int r = parse_maps(d_table, n, min_len, max_len, w, s)) { return r; }
+    if (int r = parse_maps(d_table, n, min_len, max_len, w, s, lazy)) { return r; }
     parse::chain_top<<<1, 1, 0, s>>>(w.group_map, w.groups, d_entry, entry, w.group_entry, d_result);
     LAUNCHED("chain_top");
     parse::chain_expand<<<(unsigned)((w.groups + 127) / 128), 128, 0, s>>>(
         w.exit_map, w.blocks, w.group, w.groups, w.group_entry, w.block_entry);
     LAUNCHED("chain_expand");
-    const unsigned wb = (unsigned)((w.blocks + parse::kParseWarps - 1) / parse::kParseWarps);
-    const unsigned wt = 32 * parse::kParseWarps;
     const bool small = w.pb == parse::kPBSmall;
-    if (small) {
-        parse::parse_walk<false, false, parse::kPBSmall><<<wb, wt, 0, s>>>(d_shard, d_table, n, w.blocks, min_len, w.block_entry,
-                                                                           w.count, nullptr, nullptr, 0);
-    } else {
-        parse::parse_walk<false, false, parse::kPBLarge><<<wb, wt, 0, s>>>(d_shard, d_table, n, w.blocks, min_len, w.block_entry,
-                                                                           w.count, nullptr, nullptr, 0);
+    if (lazy) {
+        return small ? parse_walks<parse::kPBSmall, true>(d_shard, d_table, n, min_len, w, d_tokens, cap, d_result, s, symbols)
+                     : parse_walks<parse::kPBLarge, true>(d_shard, d_table, n, min_len, w, d_tokens, cap, d_result, s, symbols);
     }
-    LAUNCHED("parse_count");
-    parse::scan_counts<<<1, 1024, 0, s>>>(w.count, w.blocks, w.offset, d_result);
-    LAUNCHED("scan_counts");
-#define SQZ_EMIT(SYM, PB) parse::parse_walk<true, SYM, PB><<<wb, wt, 0, s>>>(d_shard, d_table, n, w.blocks, min_len, \
-                                                                             w.block_entry, nullptr, w.offset, d_tokens, cap)
-    if (symbols) { if (small) { SQZ_EMIT(true, parse::kPBSmall); } else { SQZ_EMIT(true, parse::kPBLarge); } }
-    else         { if (small) { SQZ_EMIT(false, parse::kPBSmall); } else { SQZ_EMIT(false, parse::kPBLarge); } }
-#undef SQZ_EMIT
-    LAUNCHED("parse_emit");
-    return 0;
+    return small ? parse_walks<parse::kPBSmall, false>(d_shard, d_table, n, min_len, w, d_tokens, cap, d_result, s, symbols)
+                 : parse_walks<parse::kPBLarge, false>(d_shard, d_table, n, min_len, w, d_tokens, cap, d_result, s, symbols);
 }
 
 extern "C" int sqz_gpu_parse_device(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
@@ -1120,7 +1154,7 @@ extern "C" int sqz_gpu_parse_exit_map_device(const uint32_t* d_table, size_t n,
     if (n == 0) { return fail(EINVAL, "empty shard"); }
     cudaStream_t s = (cudaStream_t)stream;
     parse::Work w = parse::carve(d_work, n);
-    if (int r = parse_maps(d_table, n, min_len, max_len, w, s)) { return r; }
+    if (int r = parse_maps(d_table, n, min_len, max_len, w, s, false)) { return r; }
     parse::chain_total<<<1, 512, 0, s>>>(w.group_map, w.groups, max_len, d_exit_map);
     LAUNCHED("chain_total");
     return 0;
@@ -1158,6 +1192,7 @@ struct sqz_gpu_stream {
     int next_slot = 0, read_slot = 0;
     int kind = kConsumer;             // of its two stages: kTable, kTokens or kConsumer
     bool symbols = false;             // emit symbol words instead of plain tokens
+    bool lazy = false;                // parse with the lazy rule
     Stage slot[2];
     const uint64_t* prev_result = nullptr;   // device: previous chunk's result (entry hand-off)
     cudaEvent_t prev_parsed = nullptr;
@@ -1219,6 +1254,19 @@ static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* d
     // copy run beside it.
     if (int r = stage_search(s, st->data, first, n, back, ahead, st->min_len, st->max_len, st->max_dist,
                              consumer ? st->prev_tabled : nullptr)) { return r; }
+    if (st->lazy) {
+        // The lazy step at the chunk's last position reads table[n], the best match at the first position
+        // of the next chunk, which is not searched yet: that one position is searched here on its own, by
+        // the exact thread-per-position kernel.  Its look-back is the whole chunk and the halo before it;
+        // its look-ahead is the chunk's halo, which holds every byte a match there can reach.  At the end
+        // of the input table[n] is 0 (len(bytes) = 0).
+        if (ahead == 0) {
+            CU(cudaMemsetAsync(s.d_table + n, 0, 4, s.stream));
+        } else if (int r = launch_v1(s.d_data + back + n, back + n, 1, ahead - 1, st->min_len, st->max_len, st->max_dist,
+                                     s.d_table + n, s.stream)) {
+            return r;
+        }
+    }
     CU(cudaEventRecord(s.tabled, s.stream));
     st->prev_tabled = s.tabled;
     const uint8_t* d_shard = s.d_data + back;
@@ -1234,7 +1282,7 @@ static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* d
             d_entry = reinterpret_cast<const uint32_t*>(st->prev_result + 1);  // low half of overshoot
         }
         if (int r = parse_launch(d_shard, s.d_table, n, d_entry, 0, st->min_len, st->max_len,
-                                 s.d_tokens, n, s.d_work, s.d_result, late, st->symbols)) { return r; }
+                                 s.d_tokens, n, s.d_work, s.d_result, late, st->symbols, st->lazy)) { return r; }
         CU(cudaMemcpyAsync(s.h_result, s.d_result, 16, cudaMemcpyDeviceToHost, late));
         CU(cudaEventRecord(s.parsed, late));
         st->prev_parsed = s.parsed;
@@ -1310,7 +1358,7 @@ extern "C" int sqz_gpu_stream_open(sqz_gpu_stream** st, int device, const uint8_
                                    uint32_t max_len, uint32_t max_dist, size_t chunk_bytes,
                                    uint32_t flags) {
     if (st == nullptr) { return fail(EINVAL, "null stream handle"); }
-    if ((flags & ~(uint32_t)(SQZ_GPU_STREAM_SYMBOLS | SQZ_GPU_STREAM_SHORT_START)) != 0) {
+    if ((flags & ~(uint32_t)(SQZ_GPU_STREAM_SYMBOLS | SQZ_GPU_STREAM_SHORT_START | SQZ_GPU_STREAM_LAZY)) != 0) {
         return fail(EINVAL, "unknown stream flags");
     }
     if (flags & SQZ_GPU_STREAM_SYMBOLS) {
@@ -1320,6 +1368,7 @@ extern "C" int sqz_gpu_stream_open(sqz_gpu_stream** st, int device, const uint8_
     if (int r = stream_open(st, device, data, bytes, window, min_len, max_len, max_dist,
                             chunk_bytes, kConsumer, (flags & SQZ_GPU_STREAM_SHORT_START) != 0)) { return r; }
     (*st)->symbols = (flags & SQZ_GPU_STREAM_SYMBOLS) != 0;
+    (*st)->lazy = (flags & SQZ_GPU_STREAM_LAZY) != 0;
     if (bytes > 0) {
         if (int r = stream_launch_next(*st, nullptr, nullptr)) {
             sqz_gpu_stream_close(*st);
