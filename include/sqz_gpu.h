@@ -207,8 +207,12 @@ int  sqz_gpu_put_tokens(uint32_t* d_dst, size_t at, const uint32_t* d_tokens, si
  * copies are a parallel problem: a scan of the token lengths places every
  * token, every output byte starts with a hop of `dist` to its source, and
  * pointer doubling shortens all chains to one hop onto a literal.  Plain
- * tokens (not symbol words); bytes < 2 GiB per call.  EINVAL when the tokens
- * do not describe exactly `bytes` bytes or a match reaches before the start. */
+ * tokens (not symbol words): len 1..65535, dist 1..65535, whatever rules made
+ * them; bytes < 2 GiB per call.  EINVAL when bytes >= 2 GiB, when the tokens
+ * do not describe exactly `bytes` bytes, when a match reaches before the start
+ * or has dist 0, and when a literal word is not a byte value (above 0xFF, as
+ * the symbol word of a match with dist 1..4 is).  sqz_gpu_expand_tokens checks
+ * the sizes before it allocates anything.                                    */
 int sqz_gpu_expand_tokens(const uint32_t* tokens, size_t n_tokens, uint8_t* out, size_t bytes);
 /* device pointers; d_work holds sqz_gpu_expand_workspace(n_tokens, bytes) bytes.
  * Waits for the stream twice: once for the scan of the token lengths (a stream

@@ -78,7 +78,8 @@ scan_blocks(uint64_t* __restrict__ block_sum, size_t blocks, uint64_t* __restric
 
 // Every token writes its bytes' hops (and a literal its value).  One warp per 32 tokens: the
 // lanes scan their lengths, then the warp walks the 32 tokens' output range together so that
-// the stores are coalesced.
+// the stores are coalesced.  A bad token (a literal word above 0xFF, dist 0, a match reaching
+// before byte 0) raises *bad and leaves hop 0 and byte 0: garbage, but every later read is in bounds.
 __global__ void __launch_bounds__(256)
 place_tokens(const uint32_t* __restrict__ tokens, size_t n_tokens, const uint64_t* __restrict__ block_off,
              uint8_t* __restrict__ out, uint32_t* __restrict__ hop, uint64_t bytes, int* __restrict__ bad) {
@@ -125,7 +126,9 @@ place_tokens(const uint32_t* __restrict__ tokens, size_t n_tokens, const uint64_
             if (j < bytes) {
                 const uint32_t len = tk >> 16, dist = tk & 0xFFFFu;
                 if (len == 0) {
-                    out[j] = (uint8_t)tk;
+                    // a literal is a byte value: a word such as a symbol word (bits 8..15 set) is refused
+                    if (tk > 0xFFu) { *bad = 1; out[j] = 0; }
+                    else { out[j] = (uint8_t)tk; }
                     hop[j] = 0;
                 } else {
                     // a match may not reach before the start of the output (squeeze.h:529-545)

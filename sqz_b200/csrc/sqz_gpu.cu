@@ -1671,12 +1671,18 @@ extern "C" size_t sqz_gpu_expand_workspace(size_t n_tokens, size_t bytes) {
     return parse::align_up(expand_blocks(n_tokens) * 8 + 8) + 256 + parse::align_up(bytes * 4 + 4);
 }
 
-extern "C" int sqz_gpu_expand_tokens_device(const uint32_t* d_tokens, size_t n_tokens, uint8_t* d_out,
-                                            size_t bytes, void* d_work, void* stream) {
+// the sizes both expand entry points refuse before they touch the device
+static int expand_check(size_t n_tokens, size_t bytes) {
     if (bytes >= ((size_t)1 << 31)) { return fail(EINVAL, "one expand call handles less than 2 GiB"); }
     if (n_tokens > bytes) { return fail(EINVAL, "more tokens than bytes"); }
+    if (n_tokens == 0 && bytes > 0) { return fail(EINVAL, "tokens describe fewer bytes than announced"); }
+    return 0;
+}
+
+extern "C" int sqz_gpu_expand_tokens_device(const uint32_t* d_tokens, size_t n_tokens, uint8_t* d_out,
+                                            size_t bytes, void* d_work, void* stream) {
+    if (int r = expand_check(n_tokens, bytes)) { return r; }
     if (bytes == 0) { return 0; }
-    if (n_tokens == 0) { return fail(EINVAL, "tokens describe fewer bytes than announced"); }
     cudaStream_t s = (cudaStream_t)stream;
     const size_t blocks = expand_blocks(n_tokens);
     if (blocks > 0x7FFFFFFFull) { return fail(EINVAL, "too many tokens for one launch"); }
@@ -1712,12 +1718,17 @@ extern "C" int sqz_gpu_expand_tokens_device(const uint32_t* d_tokens, size_t n_t
     // garbage but in bounds: place_tokens cut every bad hop to 0.)
     CU(cudaMemcpyAsync(&h, flags, 16, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
-    if (h.bad != 0) { return fail(EINVAL, "a match reaches before the start of the output"); }
+    if (h.bad != 0) {
+        return fail(EINVAL, "a bad token: a match from before the start of the output or at distance 0, "
+                            "or a literal word above 0xFF");
+    }
     return 0;
 }
 
 extern "C" int sqz_gpu_expand_tokens(const uint32_t* tokens, size_t n_tokens, uint8_t* out, size_t bytes) {
-    if (bytes == 0) { return n_tokens == 0 ? 0 : fail(EINVAL, "tokens for an empty output"); }
+    // refused before a stream or a buffer is made: the buffers below take 5 device bytes per output byte
+    if (int r = expand_check(n_tokens, bytes)) { return r; }
+    if (bytes == 0) { return 0; }
     if (tokens == nullptr || out == nullptr) { return fail(EINVAL, "null argument"); }
     int device = -1;
     if (int r = ensure_device(device)) { return r; }
