@@ -80,6 +80,14 @@ int sqz_gpu_tokens(const uint8_t* data, size_t bytes,
                    uint32_t max_dist,
                    uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens);
 
+/* sqz_gpu_tokens with flags: 0 (the call above) or SQZ_GPU_STREAM_LAZY, the
+ * lazy parse of the token stream below, identical to what the stream delivers
+ * with that flag.  Any other bit is EINVAL.                                  */
+int sqz_gpu_tokens_ex(const uint8_t* data, size_t bytes,
+                      uint32_t window, uint32_t min_len, uint32_t max_len,
+                      uint32_t max_dist, uint32_t flags,
+                      uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens);
+
 /* The same token stream computed on several devices at once (SURVEY.md section 8e;
  * squeeze.h:345,377-394 is where the seam dependency comes from).  The input is cut
  * into n_devices contiguous shards (sizes differ by at most one byte), each uploaded
@@ -100,6 +108,19 @@ int sqz_gpu_tokens_multi(const int* devices, int n_devices,
                          uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
                          size_t* shard_tokens);
 
+/* sqz_gpu_tokens_multi with flags: 0 (the call above) or SQZ_GPU_STREAM_LAZY.
+ * The lazy step at a shard's last position reads the best match at the next
+ * shard's first position; every shard searches that one position itself from
+ * its look-ahead halo, so the seams still exchange nothing but the exit maps.
+ * The result is identical to sqz_gpu_tokens_ex() with the same flags for every
+ * n_devices.  Any other bit is EINVAL.                                       */
+int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices,
+                            const uint8_t* data, size_t bytes,
+                            uint32_t window, uint32_t min_len, uint32_t max_len,
+                            uint32_t max_dist, uint32_t flags,
+                            uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                            size_t* shard_tokens);
+
 /* Streaming form used by sqz_compress(): tokens arrive chunk by chunk, in
  * parse order, from double-buffered pinned memory while the device already
  * works on the next chunk.  *tokens stays valid until the next call.
@@ -116,9 +137,9 @@ int sqz_gpu_tokens_multi(const int* devices, int n_devices,
  * when the next position has a strictly longer match, and the decision is
  * taken again there (len at the end of the input counts as 0).  About 2 %
  * smaller streams of text and code, slightly larger ones of data that does
- * not compress; any decoder reads them.  Only this entry point has the lazy
- * parse: sqz_gpu_tokens, sqz_gpu_tokens_multi and the device-buffer parse
- * entry points below are greedy.                                            */
+ * not compress; any decoder reads them.  The same flag selects the lazy parse
+ * in sqz_gpu_tokens_ex, sqz_gpu_tokens_multi_ex and the _ex device-buffer
+ * parse entry points below; without it every entry point is greedy.         */
 typedef struct sqz_gpu_stream sqz_gpu_stream;
 #define SQZ_GPU_STREAM_SYMBOLS 1u       /* deliver symbol words instead of plain tokens */
 #define SQZ_GPU_STREAM_SHORT_START 2u   /* explicit chunk_bytes: start with chunk_bytes / 4, then / 2 */
@@ -150,6 +171,16 @@ int sqz_gpu_match_table_device_ws(const uint8_t* d_shard, size_t back, size_t n,
 int sqz_gpu_match_table_device(const uint8_t* d_shard, size_t back, size_t n,
                                size_t ahead, uint32_t min_len, uint32_t max_len,
                                uint32_t max_dist, uint32_t* d_table, void* stream);
+
+/* The seam word of a lazy parse: d_table[n] = the packed best match at the
+ * first position after the shard (position n, searched with the shard as
+ * look-back and `ahead` - 1 bytes of look-ahead), 0 when ahead is 0 (the end
+ * of the input).  A caller who searched the shard's n positions with
+ * sqz_gpu_match_table_device gets the (n+1)-th word the lazy parse reads,
+ * from the same halos; no byte beyond them is read.                          */
+int sqz_gpu_match_seam_device(const uint8_t* d_shard, size_t back, size_t n,
+                              size_t ahead, uint32_t min_len, uint32_t max_len,
+                              uint32_t max_dist, uint32_t* d_table, void* stream);
 
 /* Split a packed table into the two 16-bit arrays of sqz_gpu_match_table.   */
 int sqz_gpu_unpack_table_device(const uint32_t* d_table, size_t n,
@@ -184,6 +215,23 @@ int sqz_gpu_parse_symbols_device(const uint8_t* d_shard, const uint32_t* d_table
 int sqz_gpu_parse_exit_map_device(const uint32_t* d_table, size_t n,
                                   uint32_t min_len, uint32_t max_len,
                                   void* d_work, uint16_t* d_exit_map, void* stream);
+
+/* The three calls above with flags.  sqz_gpu_parse_device_ex takes
+ * SQZ_GPU_STREAM_SYMBOLS (symbol words, the limits of sqz_gpu_parse_symbols_device)
+ * and SQZ_GPU_STREAM_LAZY; sqz_gpu_parse_exit_map_device_ex takes
+ * SQZ_GPU_STREAM_LAZY.  Any other bit is EINVAL.  With SQZ_GPU_STREAM_LAZY
+ * d_table holds n + 1 words, the last one from sqz_gpu_match_seam_device; the
+ * entry and the overshoot stay below max_len, so the exit maps chain across
+ * shards exactly as for the greedy parse.  flags = 0 (and SYMBOLS) give the
+ * calls above.                                                               */
+int sqz_gpu_parse_device_ex(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
+                            uint32_t entry, uint32_t min_len, uint32_t max_len,
+                            uint32_t flags, uint32_t* d_out, size_t out_cap,
+                            void* d_work, uint64_t* d_result /* 2 x u64, device */,
+                            void* stream);
+int sqz_gpu_parse_exit_map_device_ex(const uint32_t* d_table, size_t n,
+                                     uint32_t min_len, uint32_t max_len, uint32_t flags,
+                                     void* d_work, uint16_t* d_exit_map, void* stream);
 
 /* ---- one process per device ------------------------------------------------ *
  * Jobs that run one process per GPU (torchrun and the like) concatenate their

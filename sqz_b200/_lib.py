@@ -82,8 +82,13 @@ SYMBOLS = {
     "sqz_gpu_match_table": (C.c_int, [u8p, size_t, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, u16p, u16p]),
     "sqz_gpu_tokens": (C.c_int, [u8p, size_t, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, u32p, size_t,
                                  C.POINTER(size_t)]),
+    "sqz_gpu_tokens_ex": (C.c_int, [u8p, size_t, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, u32p,
+                                    size_t, C.POINTER(size_t)]),
     "sqz_gpu_tokens_multi": (C.c_int, [C.POINTER(C.c_int), C.c_int, u8p, size_t, C.c_uint32, C.c_uint32, C.c_uint32,
                                        C.c_uint32, C.c_void_p, size_t, C.POINTER(size_t), C.POINTER(size_t)]),
+    "sqz_gpu_tokens_multi_ex": (C.c_int, [C.POINTER(C.c_int), C.c_int, u8p, size_t, C.c_uint32, C.c_uint32,
+                                          C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, size_t, C.POINTER(size_t),
+                                          C.POINTER(size_t)]),
     "sqz_gpu_stream_open": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, u8p, size_t, C.c_uint32, C.c_uint32,
                                       C.c_uint32, C.c_uint32, size_t, C.c_uint32]),
     "sqz_gpu_stream_next": (C.c_int, [C.c_void_p, C.POINTER(u32p), C.POINTER(size_t)]),
@@ -93,6 +98,8 @@ SYMBOLS = {
                                                 C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sqz_gpu_match_table_device": (C.c_int, [C.c_void_p, size_t, size_t, size_t, C.c_uint32, C.c_uint32,
                                              C.c_uint32, C.c_void_p, C.c_void_p]),
+    "sqz_gpu_match_seam_device": (C.c_int, [C.c_void_p, size_t, size_t, size_t, C.c_uint32, C.c_uint32,
+                                            C.c_uint32, C.c_void_p, C.c_void_p]),
     "sqz_gpu_unpack_table_device": (C.c_int, [C.c_void_p, size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sqz_gpu_parse_workspace": (size_t, [size_t]),
     "sqz_gpu_parse_device": (C.c_int, [C.c_void_p, C.c_void_p, size_t, C.c_uint32, C.c_uint32, C.c_uint32,
@@ -101,6 +108,10 @@ SYMBOLS = {
                                                C.c_void_p, size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sqz_gpu_parse_exit_map_device": (C.c_int, [C.c_void_p, size_t, C.c_uint32, C.c_uint32, C.c_void_p,
                                                 C.c_void_p, C.c_void_p]),
+    "sqz_gpu_parse_device_ex": (C.c_int, [C.c_void_p, C.c_void_p, size_t, C.c_uint32, C.c_uint32, C.c_uint32,
+                                          C.c_uint32, C.c_void_p, size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sqz_gpu_parse_exit_map_device_ex": (C.c_int, [C.c_void_p, size_t, C.c_uint32, C.c_uint32, C.c_uint32,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p]),
     "sqz_gpu_device_alloc": (C.c_int, [C.POINTER(C.c_void_p), size_t]),
     "sqz_gpu_device_free": (None, [C.c_void_p]),
     "sqz_gpu_ipc_export": (C.c_int, [C.c_void_p, C.c_char_p]),
@@ -122,6 +133,10 @@ SYMBOLS = {
     "sqz_gpu_set_timing": (None, [C.c_int]),
     "sqz_gpu_match_kernel_seconds": (C.c_double, [C.c_int, u64p]),
 }
+
+# flag bits of include/sqz_gpu.h (SQZ_GPU_STREAM_*)
+STREAM_SYMBOLS = 1
+STREAM_LAZY = 8
 
 _lib = None
 

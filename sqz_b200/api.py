@@ -78,24 +78,26 @@ def match_table(data, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len:
 
 
 def tokens(data, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len: int = G1_MAX_LEN,
-           max_dist: int | None = None) -> np.ndarray:
-    """Greedy token stream (squeeze.h:337,377-394): literal byte or (len << 16) | dist."""
+           max_dist: int | None = None, lazy: bool = False) -> np.ndarray:
+    """Token stream, greedy (squeeze.h:337,377-394; the default) or lazy: literal byte or (len << 16) | dist.
+    lazy=True parses with lazy matching (sqz_gpu_tokens_ex with SQZ_GPU_STREAM_LAZY): the
+    tokens sq.compress(data, lazy=True) codes."""
     L = _lib.load()
     d = _u8(data)
     w, lo, hi, md = _rules(window, min_len, max_len, max_dist)
     out = np.empty(max(d.size, 1), dtype=np.uint32)
     n = C.c_size_t()
-    rc = L.sqz_gpu_tokens(d.ctypes.data_as(u8p), d.size, w, lo, hi, md,
-                          out.ctypes.data_as(u32p), out.size, C.byref(n))
-    _check(rc, "sqz_gpu_tokens")
+    rc = L.sqz_gpu_tokens_ex(d.ctypes.data_as(u8p), d.size, w, lo, hi, md, _lib.STREAM_LAZY if lazy else 0,
+                             out.ctypes.data_as(u32p), out.size, C.byref(n))
+    _check(rc, "sqz_gpu_tokens_ex")
     return out[: n.value].copy()
 
 
 def tokens_multi(data, devices, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len: int = G1_MAX_LEN,
-                 max_dist: int | None = None, return_shard_counts: bool = False):
-    """The same token stream computed on several GPUs of this process (sqz_gpu_tokens_multi):
+                 max_dist: int | None = None, return_shard_counts: bool = False, lazy: bool = False):
+    """The same token stream computed on several GPUs of this process (sqz_gpu_tokens_multi_ex):
     contiguous shards with halos, seams chained on the host, token arrays concatenated in shard
-    order by copies sized by their counts.  Identical to tokens() for every device list."""
+    order by copies sized by their counts.  Identical to tokens(lazy=lazy) for every device list."""
     L = _lib.load()
     d = _u8(data)
     w, lo, hi, md = _rules(window, min_len, max_len, max_dist)
@@ -103,9 +105,9 @@ def tokens_multi(data, devices, window: int = 1 << 15, min_len: int = G1_MIN_LEN
     out = np.empty(max(d.size, 1), dtype=np.uint32)
     n = C.c_size_t()
     per = (C.c_size_t * len(devices))()
-    rc = L.sqz_gpu_tokens_multi(devs, len(devices), d.ctypes.data_as(u8p), d.size, w, lo, hi, md,
-                                out.ctypes.data, out.size, C.byref(n), per)
-    _check(rc, "sqz_gpu_tokens_multi")
+    rc = L.sqz_gpu_tokens_multi_ex(devs, len(devices), d.ctypes.data_as(u8p), d.size, w, lo, hi, md,
+                                   _lib.STREAM_LAZY if lazy else 0, out.ctypes.data, out.size, C.byref(n), per)
+    _check(rc, "sqz_gpu_tokens_multi_ex")
     t = out[: n.value].copy()
     return (t, [int(x) for x in per]) if return_shard_counts else t
 

@@ -7,8 +7,8 @@
 // Results are bit-exact: for every position the longest common prefix with a
 // candidate at distance 1..max_dist (capped by max_len and the end of data),
 // the nearest candidate among equals; then the orbit of position 0 under
-// next[i] = i + (len[i] >= min_len ? len[i] : 1) as the token stream.  The streaming
-// pipeline can parse with lazy matching instead (SQZ_GPU_STREAM_LAZY, namespace parse).
+// next[i] = i + (len[i] >= min_len ? len[i] : 1) as the token stream.  Every token entry
+// point can parse with lazy matching instead (SQZ_GPU_STREAM_LAZY, namespace parse).
 //
 // There is no CPU fallback in this file: without a device every entry point
 // returns ENODEV.
@@ -892,6 +892,21 @@ static int launch_v1(const uint8_t* d_shard, size_t back, size_t n, size_t ahead
     return 0;
 }
 
+// The seam word of a lazy parse: the lazy step at a shard's last position reads table[n], the best match
+// at the first position after the shard, which belongs to the next shard (or chunk) and is searched there
+// only later, if at all.  That one position is searched here on its own, by the exact thread-per-position
+// kernel.  Its look-back is the shard and the halo before it; its look-ahead is the shard's own halo, which
+// holds every byte a match there can reach (min(rest, max_len) bytes).  At the end of the input
+// (ahead = 0) table[n] is 0: len(bytes) = 0.  The same halos as the shard's table search, nothing more.
+static int seam_word(const uint8_t* d_shard, size_t back, size_t n, size_t ahead, uint32_t min_len,
+                     uint32_t max_len, uint32_t max_dist, uint32_t* d_table, cudaStream_t s) {
+    if (ahead == 0) {
+        CU(cudaMemsetAsync(d_table + n, 0, 4, s));
+        return 0;
+    }
+    return launch_v1(d_shard + n, back + n, 1, ahead - 1, min_len, max_len, max_dist, d_table + n, s);
+}
+
 template <int kMinLen, int kQ>
 static int launch_tiles(const SlicePlan& sp, const uint8_t* d_shard, size_t back, size_t n, size_t ahead, uint32_t max_len,
                         uint32_t max_dist, uint32_t* d_table, void* d_work, cudaStream_t s) {
@@ -1037,6 +1052,13 @@ extern "C" int sqz_gpu_match_table_device(const uint8_t* d_shard, size_t back, s
     return r;
 }
 
+extern "C" int sqz_gpu_match_seam_device(const uint8_t* d_shard, size_t back, size_t n, size_t ahead,
+                                         uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                                         uint32_t* d_table, void* stream) {
+    if (int r = check_rules(min_len, max_len, max_dist)) { return r; }
+    return seam_word(d_shard, back, n, ahead, min_len, max_len, max_dist, d_table, (cudaStream_t)stream);
+}
+
 extern "C" int sqz_gpu_unpack_table_device(const uint32_t* d_table, size_t n,
                                            uint16_t* d_len, uint16_t* d_dist, void* stream) {
     if (n == 0) { return 0; }
@@ -1116,16 +1138,6 @@ static int parse_launch(const uint8_t* d_shard, const uint32_t* d_table, size_t 
                  : parse_walks<parse::kPBLarge, false>(d_shard, d_table, n, min_len, w, d_tokens, cap, d_result, s, symbols);
 }
 
-extern "C" int sqz_gpu_parse_device(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
-                                    uint32_t entry, uint32_t min_len, uint32_t max_len,
-                                    uint32_t* d_tokens, size_t tokens_cap, void* d_work,
-                                    uint64_t* d_result, void* stream) {
-    if (int r = check_rules(min_len, max_len, 1)) { return r; }
-    if (entry >= max_len) { return fail(EINVAL, "entry must be < max_len"); }
-    return parse_launch(d_shard, d_table, n, nullptr, entry, min_len, max_len, d_tokens,
-                        tokens_cap, d_work, d_result, (cudaStream_t)stream);
-}
-
 // symbol words only exist for the bitstream's own limits (squeeze.h:13-15, 529-545)
 static int check_symbol_rules(uint32_t min_len, uint32_t max_len, uint32_t max_dist) {
     // 258 has a bucket (27, extra bits 31) but no decoder accepts it: squeeze.h:529-545 and
@@ -1136,28 +1148,61 @@ static int check_symbol_rules(uint32_t min_len, uint32_t max_len, uint32_t max_d
     return 0;
 }
 
+// the flag bits an entry point takes (SQZ_GPU_STREAM_*); any other bit is EINVAL
+static int check_flags(uint32_t flags, uint32_t allowed) {
+    if ((flags & ~allowed) != 0) { return fail(EINVAL, "flag bits this entry point does not take"); }
+    return 0;
+}
+
+extern "C" int sqz_gpu_parse_device_ex(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
+                                       uint32_t entry, uint32_t min_len, uint32_t max_len, uint32_t flags,
+                                       uint32_t* d_out, size_t out_cap, void* d_work,
+                                       uint64_t* d_result, void* stream) {
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY | SQZ_GPU_STREAM_SYMBOLS)) { return r; }
+    const bool symbols = (flags & SQZ_GPU_STREAM_SYMBOLS) != 0;
+    if (int r = check_rules(min_len, max_len, 1)) { return r; }
+    if (symbols) {
+        if (int r = check_symbol_rules(min_len, max_len, 1)) { return r; }
+    }
+    if (entry >= max_len) { return fail(EINVAL, "entry must be < max_len"); }
+    return parse_launch(d_shard, d_table, n, nullptr, entry, min_len, max_len, d_out, out_cap, d_work, d_result,
+                        (cudaStream_t)stream, symbols, (flags & SQZ_GPU_STREAM_LAZY) != 0);
+}
+
+extern "C" int sqz_gpu_parse_device(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
+                                    uint32_t entry, uint32_t min_len, uint32_t max_len,
+                                    uint32_t* d_tokens, size_t tokens_cap, void* d_work,
+                                    uint64_t* d_result, void* stream) {
+    return sqz_gpu_parse_device_ex(d_shard, d_table, n, entry, min_len, max_len, 0, d_tokens, tokens_cap, d_work,
+                                   d_result, stream);
+}
+
 extern "C" int sqz_gpu_parse_symbols_device(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
                                             uint32_t entry, uint32_t min_len, uint32_t max_len,
                                             uint32_t* d_words, size_t words_cap, void* d_work,
                                             uint64_t* d_result, void* stream) {
+    return sqz_gpu_parse_device_ex(d_shard, d_table, n, entry, min_len, max_len, SQZ_GPU_STREAM_SYMBOLS, d_words,
+                                   words_cap, d_work, d_result, stream);
+}
+
+extern "C" int sqz_gpu_parse_exit_map_device_ex(const uint32_t* d_table, size_t n, uint32_t min_len,
+                                                uint32_t max_len, uint32_t flags, void* d_work,
+                                                uint16_t* d_exit_map, void* stream) {
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY)) { return r; }
     if (int r = check_rules(min_len, max_len, 1)) { return r; }
-    if (int r = check_symbol_rules(min_len, max_len, 1)) { return r; }
-    if (entry >= max_len) { return fail(EINVAL, "entry must be < max_len"); }
-    return parse_launch(d_shard, d_table, n, nullptr, entry, min_len, max_len, d_words,
-                        words_cap, d_work, d_result, (cudaStream_t)stream, true);
+    if (n == 0) { return fail(EINVAL, "empty shard"); }
+    cudaStream_t s = (cudaStream_t)stream;
+    parse::Work w = parse::carve(d_work, n);
+    if (int r = parse_maps(d_table, n, min_len, max_len, w, s, (flags & SQZ_GPU_STREAM_LAZY) != 0)) { return r; }
+    parse::chain_total<<<1, 512, 0, s>>>(w.group_map, w.groups, max_len, d_exit_map);
+    LAUNCHED("chain_total");
+    return 0;
 }
 
 extern "C" int sqz_gpu_parse_exit_map_device(const uint32_t* d_table, size_t n,
                                              uint32_t min_len, uint32_t max_len, void* d_work,
                                              uint16_t* d_exit_map, void* stream) {
-    if (int r = check_rules(min_len, max_len, 1)) { return r; }
-    if (n == 0) { return fail(EINVAL, "empty shard"); }
-    cudaStream_t s = (cudaStream_t)stream;
-    parse::Work w = parse::carve(d_work, n);
-    if (int r = parse_maps(d_table, n, min_len, max_len, w, s, false)) { return r; }
-    parse::chain_total<<<1, 512, 0, s>>>(w.group_map, w.groups, max_len, d_exit_map);
-    LAUNCHED("chain_total");
-    return 0;
+    return sqz_gpu_parse_exit_map_device_ex(d_table, n, min_len, max_len, 0, d_work, d_exit_map, stream);
 }
 
 // ---------------------------------------------------------------------------
@@ -1254,18 +1299,9 @@ static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* d
     // copy run beside it.
     if (int r = stage_search(s, st->data, first, n, back, ahead, st->min_len, st->max_len, st->max_dist,
                              consumer ? st->prev_tabled : nullptr)) { return r; }
-    if (st->lazy) {
-        // The lazy step at the chunk's last position reads table[n], the best match at the first position
-        // of the next chunk, which is not searched yet: that one position is searched here on its own, by
-        // the exact thread-per-position kernel.  Its look-back is the whole chunk and the halo before it;
-        // its look-ahead is the chunk's halo, which holds every byte a match there can reach.  At the end
-        // of the input table[n] is 0 (len(bytes) = 0).
-        if (ahead == 0) {
-            CU(cudaMemsetAsync(s.d_table + n, 0, 4, s.stream));
-        } else if (int r = launch_v1(s.d_data + back + n, back + n, 1, ahead - 1, st->min_len, st->max_len, st->max_dist,
-                                     s.d_table + n, s.stream)) {
-            return r;
-        }
+    if (st->lazy) {                     // table[n]: the next chunk is not searched yet
+        if (int r = seam_word(s.d_data + back, back, n, ahead, st->min_len, st->max_len, st->max_dist,
+                              s.d_table, s.stream)) { return r; }
     }
     CU(cudaEventRecord(s.tabled, s.stream));
     st->prev_tabled = s.tabled;
@@ -1421,17 +1457,20 @@ extern "C" void sqz_gpu_stream_close(sqz_gpu_stream* st) {
 // One-shot token call: the chunks' tokens go straight from device memory to their final place in
 // the caller's buffer, count x 4 bytes each (a pinned destination takes them by DMA while the next
 // chunk is searched; a pageable one through the driver's staging).  Nothing consumes the chunks
-// on the way, so the larger streaming chunk is used.
-extern "C" int sqz_gpu_tokens(const uint8_t* data, size_t bytes, uint32_t window,
-                              uint32_t min_len, uint32_t max_len, uint32_t max_dist,
-                              uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens) {
+// on the way, so the larger streaming chunk is used.  The lazy parse crosses its chunk seams as in the
+// token stream: every chunk searches its seam word.
+extern "C" int sqz_gpu_tokens_ex(const uint8_t* data, size_t bytes, uint32_t window,
+                                 uint32_t min_len, uint32_t max_len, uint32_t max_dist, uint32_t flags,
+                                 uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens) {
     if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
     *n_tokens = 0;
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY)) { return r; }
     sqz_gpu_stream* st = nullptr;
     DeviceScope keep;
     if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kTokens)) {
         return r;
     }
+    st->lazy = (flags & SQZ_GPU_STREAM_LAZY) != 0;
     size_t total = 0;
     int rc = 0;
     if (bytes > 0) { rc = stream_launch_next(st, nullptr, nullptr); }
@@ -1469,6 +1508,12 @@ extern "C" int sqz_gpu_tokens(const uint8_t* data, size_t bytes, uint32_t window
     return rc;
 }
 
+extern "C" int sqz_gpu_tokens(const uint8_t* data, size_t bytes, uint32_t window,
+                              uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                              uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens) {
+    return sqz_gpu_tokens_ex(data, bytes, window, min_len, max_len, max_dist, 0, tokens_out, tokens_cap, n_tokens);
+}
+
 extern "C" int sqz_gpu_match_table(const uint8_t* data, size_t bytes, uint32_t window,
                                    uint32_t min_len, uint32_t max_len, uint32_t max_dist,
                                    uint16_t* len_out, uint16_t* dist_out) {
@@ -1502,13 +1547,15 @@ extern "C" int sqz_gpu_match_table(const uint8_t* data, size_t bytes, uint32_t w
 // 1 KiB), the host chains the maps (one lookup per seam), every device then emits its tokens from
 // its true entry, and the token arrays are concatenated in shard order by plain copies sized by
 // their counts: device -> host when tokens_out is host memory, peer-to-peer (cudaMemcpyPeerAsync
-// over NVLink) when it is device memory.
+// over NVLink) when it is device memory.  The lazy parse adds one dependency per seam, the best match
+// at the next shard's first position (table[n]), which every shard searches from its own halos: no
+// exchange beyond the exit maps.
 // ---------------------------------------------------------------------------
 static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_t* data, size_t bytes,
-                     uint32_t min_len, uint32_t max_len, uint32_t max_dist, uint32_t* tokens_out,
+                     uint32_t min_len, uint32_t max_len, uint32_t max_dist, bool lazy, uint32_t* tokens_out,
                      size_t tokens_cap, bool out_on_device, int out_device, size_t* n_tokens,
                      size_t* shard_tokens) {
-    // phase A on every device at once: upload, match table, composed exit map
+    // phase A on every device at once: upload, match table (and the seam word), composed exit map
     const size_t base = bytes / parts.size(), extra = bytes % parts.size();
     size_t first = 0;
     for (size_t g = 0; g < parts.size(); g++) {
@@ -1517,10 +1564,14 @@ static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_
             Stage& p = parts[g];
             CU(cudaSetDevice(devices[g]));
             if (int r = stage_take(p, devices[g], kTokens, n)) { return r; }
-            if (int r = stage_search(p, data, first, n, std::min<size_t>(first, max_dist),
-                                     std::min<size_t>(bytes - (first + n), max_len), min_len, max_len, max_dist,
-                                     nullptr)) { return r; }
-            if (int r = sqz_gpu_parse_exit_map_device(p.d_table, n, min_len, max_len, p.d_work, p.d_map, p.stream)) { return r; }
+            const size_t back = std::min<size_t>(first, max_dist), ahead = std::min<size_t>(bytes - (first + n), max_len);
+            if (int r = stage_search(p, data, first, n, back, ahead, min_len, max_len, max_dist, nullptr)) { return r; }
+            if (lazy) {
+                if (int r = seam_word(p.d_data + back, back, n, ahead, min_len, max_len, max_dist, p.d_table,
+                                      p.stream)) { return r; }
+            }
+            if (int r = sqz_gpu_parse_exit_map_device_ex(p.d_table, n, min_len, max_len, lazy ? SQZ_GPU_STREAM_LAZY : 0,
+                                                         p.d_work, p.d_map, p.stream)) { return r; }
             CU(cudaMemcpyAsync(p.h_map, p.d_map, (size_t)max_len * 2, cudaMemcpyDeviceToHost, p.stream));
             CU(cudaEventRecord(p.tabled, p.stream));
         }
@@ -1535,7 +1586,7 @@ static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_
         if (entry >= max_len) { return fail(EIO, "seam entry out of range"); }
         const uint32_t next_entry = p.h_map[entry];
         if (int r = parse_launch(p.d_data + p.back, p.d_table, p.n, nullptr, entry, min_len, max_len, p.d_tokens,
-                                 p.n, p.d_work, p.d_result, p.stream)) { return r; }
+                                 p.n, p.d_work, p.d_result, p.stream, false, lazy)) { return r; }
         CU(cudaMemcpyAsync(p.h_result, p.d_result, 16, cudaMemcpyDeviceToHost, p.stream));
         CU(cudaEventRecord(p.parsed, p.stream));
         entry = next_entry;
@@ -1567,12 +1618,13 @@ static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_
     return total > tokens_cap ? fail(E2BIG, "token buffer too small") : 0;
 }
 
-extern "C" int sqz_gpu_tokens_multi(const int* devices, int n_devices, const uint8_t* data, size_t bytes,
-                                    uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
-                                    uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
-                                    size_t* shard_tokens) {
+extern "C" int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices, const uint8_t* data, size_t bytes,
+                                       uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                                       uint32_t flags, uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                                       size_t* shard_tokens) {
     if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
     *n_tokens = 0;
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY)) { return r; }
     if (devices == nullptr || n_devices < 1 || n_devices > kMaxDevices) { return fail(EINVAL, "bad device list"); }
     DeviceScope keep;
     int device = devices[0];
@@ -1607,10 +1659,18 @@ extern "C" int sqz_gpu_tokens_multi(const int* devices, int n_devices, const uin
         }
     }
     std::vector<Stage> parts((size_t)n_devices);
-    int rc = multi_run(parts, devices, data, bytes, min_len, max_len, max_dist, tokens_out, tokens_cap,
-                       out_on_device, out_device, n_tokens, shard_tokens);
+    int rc = multi_run(parts, devices, data, bytes, min_len, max_len, max_dist, (flags & SQZ_GPU_STREAM_LAZY) != 0,
+                       tokens_out, tokens_cap, out_on_device, out_device, n_tokens, shard_tokens);
     for (Stage& p : parts) { rc = stage_finish(p, rc); }
     return rc;
+}
+
+extern "C" int sqz_gpu_tokens_multi(const int* devices, int n_devices, const uint8_t* data, size_t bytes,
+                                    uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                                    uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                                    size_t* shard_tokens) {
+    return sqz_gpu_tokens_multi_ex(devices, n_devices, data, bytes, window, min_len, max_len, max_dist, 0, tokens_out,
+                                   tokens_cap, n_tokens, shard_tokens);
 }
 
 // ---------------------------------------------------------------------------

@@ -27,47 +27,60 @@ def _need(t: torch.Tensor, what: str, dtype, numel: int, device) -> None:
 
 
 def match_table(buf: torch.Tensor, first: int, n: int, back: int, ahead: int, min_len: int = G1_MIN_LEN,
-                max_len: int = G1_MAX_LEN, max_dist: int = (1 << 15) - 1, out: torch.Tensor | None = None) -> torch.Tensor:
-    """Packed table words (len << 16 | dist) for buf[first : first+n]  (squeeze.h:340-358 at every i)."""
+                max_len: int = G1_MAX_LEN, max_dist: int = (1 << 15) - 1, out: torch.Tensor | None = None,
+                seam: bool = False) -> torch.Tensor:
+    """Packed table words (len << 16 | dist) for buf[first : first+n]  (squeeze.h:340-358 at every i).
+    seam=True: n + 1 words, the last one the seam word a lazy parse of the shard reads (the best match at
+    first + n from the same halos, 0 at the end of the input; sqz_gpu_match_seam_device)."""
     _need(buf, "buf", torch.uint8, first + n + ahead, buf.device if isinstance(buf, torch.Tensor) else None)
     if first - back < 0 or n < 0:
         raise ValueError("the look-back halo reaches before the buffer")
+    words = n + 1 if seam else n
     if out is None:
-        out = torch.empty(max(n, 1), dtype=torch.int32, device=buf.device)
+        out = torch.empty(max(words, 1), dtype=torch.int32, device=buf.device)
     else:
-        _need(out, "out", torch.int32, n, buf.device)
-    rc = _lib.load().sqz_gpu_match_table_device(buf.data_ptr() + first, back, n, ahead, min_len, max_len, max_dist,
-                                                out.data_ptr(), _stream())
-    _check(rc, "sqz_gpu_match_table_device")
-    return out[:n]
-
-
-def exit_map(table: torch.Tensor, n: int, min_len: int = G1_MIN_LEN, max_len: int = G1_MAX_LEN) -> torch.Tensor:
-    """exit_map[e] = overshoot of the shard when entered at offset e (512 x int16 on the device)."""
+        _need(out, "out", torch.int32, words, buf.device)
     L = _lib.load()
-    _need(table, "table", torch.int32, n, table.device if isinstance(table, torch.Tensor) else None)
+    rc = L.sqz_gpu_match_table_device(buf.data_ptr() + first, back, n, ahead, min_len, max_len, max_dist,
+                                      out.data_ptr(), _stream())
+    _check(rc, "sqz_gpu_match_table_device")
+    if seam:
+        rc = L.sqz_gpu_match_seam_device(buf.data_ptr() + first, back, n, ahead, min_len, max_len, max_dist,
+                                         out.data_ptr(), _stream())
+        _check(rc, "sqz_gpu_match_seam_device")
+    return out[:words]
+
+
+def exit_map(table: torch.Tensor, n: int, min_len: int = G1_MIN_LEN, max_len: int = G1_MAX_LEN,
+             lazy: bool = False) -> torch.Tensor:
+    """exit_map[e] = overshoot of the shard when entered at offset e (512 x int16 on the device).
+    lazy=True: of the lazy parse, whose table holds n + 1 words (match_table(..., seam=True))."""
+    L = _lib.load()
+    _need(table, "table", torch.int32, n + 1 if lazy else n, table.device if isinstance(table, torch.Tensor) else None)
     work = torch.empty(L.sqz_gpu_parse_workspace(n), dtype=torch.uint8, device=table.device)
     out = torch.zeros(512, dtype=torch.int16, device=table.device)
-    rc = L.sqz_gpu_parse_exit_map_device(table.data_ptr(), n, min_len, max_len, work.data_ptr(), out.data_ptr(), _stream())
-    _check(rc, "sqz_gpu_parse_exit_map_device")
+    rc = L.sqz_gpu_parse_exit_map_device_ex(table.data_ptr(), n, min_len, max_len, _lib.STREAM_LAZY if lazy else 0,
+                                            work.data_ptr(), out.data_ptr(), _stream())
+    _check(rc, "sqz_gpu_parse_exit_map_device_ex")
     torch.cuda.current_stream().synchronize()      # `work` must outlive the kernels
     return out
 
 
 def parse(buf: torch.Tensor, first: int, table: torch.Tensor, n: int, entry: int = 0, min_len: int = G1_MIN_LEN,
-          max_len: int = G1_MAX_LEN, symbols: bool = False):
-    """Greedy parse of one shard (squeeze.h:337,377-394): (tokens int32[count], overshoot).
-    symbols=True: symbol words (include/sqz_gpu.h) instead of plain tokens."""
+          max_len: int = G1_MAX_LEN, symbols: bool = False, lazy: bool = False):
+    """Greedy (squeeze.h:337,377-394; the default) or lazy parse of one shard: (tokens int32[count], overshoot).
+    symbols=True: symbol words (include/sqz_gpu.h) instead of plain tokens.  lazy=True: the lazy parse,
+    whose table holds n + 1 words (match_table(..., seam=True))."""
     L = _lib.load()
     dev = buf.device if isinstance(buf, torch.Tensor) else None
     _need(buf, "buf", torch.uint8, first + n, dev)
-    _need(table, "table", torch.int32, n, dev)
+    _need(table, "table", torch.int32, n + 1 if lazy else n, dev)
     work = torch.empty(L.sqz_gpu_parse_workspace(n), dtype=torch.uint8, device=dev)
     tokens = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
     result = torch.zeros(2, dtype=torch.int64, device=dev)
-    fn = L.sqz_gpu_parse_symbols_device if symbols else L.sqz_gpu_parse_device
-    rc = fn(buf.data_ptr() + first, table.data_ptr(), n, entry, min_len, max_len,
-            tokens.data_ptr(), n, work.data_ptr(), result.data_ptr(), _stream())
-    _check(rc, "sqz_gpu_parse_symbols_device" if symbols else "sqz_gpu_parse_device")
+    flags = (_lib.STREAM_SYMBOLS if symbols else 0) | (_lib.STREAM_LAZY if lazy else 0)
+    rc = L.sqz_gpu_parse_device_ex(buf.data_ptr() + first, table.data_ptr(), n, entry, min_len, max_len, flags,
+                                   tokens.data_ptr(), n, work.data_ptr(), result.data_ptr(), _stream())
+    _check(rc, "sqz_gpu_parse_device_ex")
     count, overshoot = (int(x) for x in result.cpu())
     return tokens[:count], overshoot

@@ -7,6 +7,12 @@ has one scalar dependency per seam: the first parse position of shard g+1 is the
 overshoot of shard g's last token.  Every shard publishes exit_map[e] = "overshoot I
 produce when entered at offset e" (sqz_gpu_parse_exit_map_device); chaining those maps
 gives every shard its true entry after one tiny all-gather.
+
+Nothing here depends on the parse rule.  The lazy parse steps 1 or len <= max_len as well, so
+entries and overshoots keep their bounds; its one extra input at a seam, the best match at the
+next shard's first position, every shard searches itself from its own look-ahead halo
+(device.match_table(..., seam=True)), and its maps (device.exit_map(..., lazy=True)) chain here
+unchanged.
 """
 from __future__ import annotations
 
