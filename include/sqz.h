@@ -113,7 +113,12 @@ struct sqz {
     uint8_t len_index[sqz_max_len + 2]; /* len -> length bucket, squeeze.h:151-161.  Also keeps the two tree
                                            headers on different cache lines: with two coder threads each
                                            tree's counters are written by another thread for every token */
-    uint8_t apart[64];
+    int32_t mincost;                    /* sqz_compress's parse: 0 (sqz_init) = as `lazy` says; 1 = the min-cost
+                                           parse (SQZ_GPU_STREAM_MINCOST in sqz_gpu.h): 3-5 % smaller than greedy
+                                           on text and code, the same on data that does not compress, read by
+                                           every decoder; other values, and 1 with lazy = 1: EINVAL.  (It takes
+                                           the first four bytes of what was apart[64]: same size and offsets.) */
+    uint8_t apart[60];
     struct sqz_tree pos;
     SQZ_TREE_STORE(sqz_lit_symbols) lit_store;
     SQZ_TREE_STORE(sqz_pos_symbols) pos_store;
@@ -131,7 +136,7 @@ void sqz_read_header(struct sqz_bitstream* bs, uint64_t* bytes, uint8_t* win_bit
 void sqz_init(struct sqz* s);
 
 /* LZ77 (GPU) + adaptive Huffman (host).  window must be a power of two in
- * [2^10, 2^15].  The parse is greedy unless s->lazy is 1.  Errors are
+ * [2^10, 2^15].  The parse is greedy unless s->lazy or s->mincost is 1.  Errors are
  * reported in s->error.                                                      */
 void sqz_compress(struct sqz* s, struct sqz_bitstream* bs,
                   const uint8_t* data, uint64_t bytes, uint32_t window);

@@ -55,7 +55,7 @@ class State(C.Structure):
         ("tokens", C.c_uint64), ("matches", C.c_uint64),
         ("search_seconds", C.c_double), ("entropy_seconds", C.c_double),
         ("coder_threads", C.c_int32), ("lazy", C.c_int32),
-        ("lit", Tree), ("len_index", C.c_uint8 * 259), ("apart", C.c_uint8 * 64), ("pos", Tree),
+        ("lit", Tree), ("len_index", C.c_uint8 * 259), ("mincost", C.c_int32), ("apart", C.c_uint8 * 60), ("pos", Tree),
         ("lit_store", _store(512)), ("pos_store", _store(32)),
         ("lit_lut", C.c_uint16 * 1024), ("pos_lut", C.c_uint16 * 64),
     ]
@@ -132,11 +132,13 @@ SYMBOLS = {
     "sqz_gpu_launch_count": (C.c_uint64, []),
     "sqz_gpu_set_timing": (None, [C.c_int]),
     "sqz_gpu_match_kernel_seconds": (C.c_double, [C.c_int, u64p]),
+    "sqz_gpu_mincost_kernel_seconds": (C.c_double, [C.c_int, u64p]),
 }
 
 # flag bits of include/sqz_gpu.h (SQZ_GPU_STREAM_*)
 STREAM_SYMBOLS = 1
 STREAM_LAZY = 8
+STREAM_MINCOST = 32
 
 _lib = None
 

@@ -77,17 +77,24 @@ def match_table(data, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len:
     return ln, ds
 
 
+def _parse_flags(lazy: bool, mincost: bool) -> int:
+    if lazy and mincost:
+        raise ValueError("lazy and mincost are two different parses: choose one")
+    return (_lib.STREAM_LAZY if lazy else 0) | (_lib.STREAM_MINCOST if mincost else 0)
+
+
 def tokens(data, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len: int = G1_MAX_LEN,
-           max_dist: int | None = None, lazy: bool = False) -> np.ndarray:
-    """Token stream, greedy (squeeze.h:337,377-394; the default) or lazy: literal byte or (len << 16) | dist.
-    lazy=True parses with lazy matching (sqz_gpu_tokens_ex with SQZ_GPU_STREAM_LAZY): the
-    tokens sq.compress(data, lazy=True) codes."""
+           max_dist: int | None = None, lazy: bool = False, mincost: bool = False) -> np.ndarray:
+    """Token stream, greedy (squeeze.h:337,377-394; the default), lazy or min-cost: literal byte or
+    (len << 16) | dist.  lazy=True parses with lazy matching (sqz_gpu_tokens_ex with SQZ_GPU_STREAM_LAZY):
+    the tokens sq.compress(data, lazy=True) codes.  mincost=True parses by cost (SQZ_GPU_STREAM_MINCOST,
+    within the bitstream's limits only): the tokens sq.compress(data, mincost=True) codes."""
     L = _lib.load()
     d = _u8(data)
     w, lo, hi, md = _rules(window, min_len, max_len, max_dist)
     out = np.empty(max(d.size, 1), dtype=np.uint32)
     n = C.c_size_t()
-    rc = L.sqz_gpu_tokens_ex(d.ctypes.data_as(u8p), d.size, w, lo, hi, md, _lib.STREAM_LAZY if lazy else 0,
+    rc = L.sqz_gpu_tokens_ex(d.ctypes.data_as(u8p), d.size, w, lo, hi, md, _parse_flags(lazy, mincost),
                              out.ctypes.data_as(u32p), out.size, C.byref(n))
     _check(rc, "sqz_gpu_tokens_ex")
     return out[: n.value].copy()
@@ -125,12 +132,14 @@ def _capacity(nbytes: int) -> int:
 
 
 def compress(data, win_bits: int = 15, file_mode: bool = False, stats: dict | None = None,
-             threads: int = 0, into=None, lazy: bool = False):
+             threads: int = 0, into=None, lazy: bool = False, mincost: bool = False):
     """squeeze.write_header + squeeze.compress: GPU search, host entropy stage.  Returns the bitstream as
     bytes -- or, with `into` (a C-contiguous writable uint8 array of at least capacity(len(data)) bytes, the
     caller's buffer as in the C API), a view of the part of it that was written, without a copy.
     lazy=True parses with lazy matching (struct sqz's `lazy`): a smaller stream on text and code, in the
-    same format; the default greedy parse gives the reference's exact bytes."""
+    same format; the default greedy parse gives the reference's exact bytes.  mincost=True (struct sqz's
+    `mincost`) parses by cost: smaller still on text and code, also in the same format.  Not both."""
+    _parse_flags(lazy, mincost)
     L = _lib.load()
     d = _u8(data)
     if into is not None:
@@ -160,6 +169,7 @@ def compress(data, win_bits: int = 15, file_mode: bool = False, stats: dict | No
     L.sqz_init(C.byref(s))
     s.coder_threads = threads
     s.lazy = 1 if lazy else 0
+    s.mincost = 1 if mincost else 0
     L.sqz_compress(C.byref(s), C.byref(bs), d.ctypes.data_as(u8p), d.size, 1 << win_bits)
     _check(s.error, "sqz_compress")
     if stats is not None:

@@ -2255,13 +2255,14 @@ void sqz_encode_symbols_chunked(struct sqz* s, struct sqz_bitstream* bs,
 void sqz_compress(struct sqz* s, struct sqz_bitstream* bs,
                   const uint8_t* data, uint64_t bytes, uint32_t window) {
     if (window < (1u << sqz_min_win_bits) || window > (1u << sqz_max_win_bits) ||
-        (window & (window - 1)) != 0 || (s->lazy != 0 && s->lazy != 1)) {
+        (window & (window - 1)) != 0 || (s->lazy != 0 && s->lazy != 1) ||
+        (s->mincost != 0 && s->mincost != 1) || (s->lazy == 1 && s->mincost == 1)) {
         s->error = EINVAL;
         return;
     }
     coder_begin(s, bs);
     if (s->error != 0) { return; }
-    /* The GPU produces the token stream (greedy, or lazy) chunk by chunk, as symbol words;
+    /* The GPU produces the token stream (greedy, lazy or min-cost) chunk by chunk, as symbol words;
      * while the host entropy-codes chunk k the device already searches chunk k+1. */
     sqz_gpu_stream* st = NULL;
     double t_search = 0, t_code = 0, t0 = now_seconds();
@@ -2278,7 +2279,8 @@ void sqz_compress(struct sqz* s, struct sqz_bitstream* bs,
     int r = sqz_gpu_stream_open(&st, s->device, data, (size_t)bytes, window,
                                 sqz_min_len, sqz_max_len, window - 1, chunk,
                                 SQZ_GPU_STREAM_SYMBOLS | (chunk != 0 ? SQZ_GPU_STREAM_SHORT_START : 0) |
-                                (s->lazy == 1 ? SQZ_GPU_STREAM_LAZY : 0));
+                                (s->lazy == 1 ? SQZ_GPU_STREAM_LAZY : 0) |
+                                (s->mincost == 1 ? SQZ_GPU_STREAM_MINCOST : 0));
     t_search += now_seconds() - t0;
     if (r != 0) { s->error = r; return; }
     struct team run;

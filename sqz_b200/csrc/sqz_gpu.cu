@@ -8,7 +8,8 @@
 // candidate at distance 1..max_dist (capped by max_len and the end of data),
 // the nearest candidate among equals; then the orbit of position 0 under
 // next[i] = i + (len[i] >= min_len ? len[i] : 1) as the token stream.  Every token entry
-// point can parse with lazy matching instead (SQZ_GPU_STREAM_LAZY, namespace parse).
+// point can parse with lazy matching instead (SQZ_GPU_STREAM_LAZY, namespace parse); the token
+// stream and the one-shot call can parse by cost (SQZ_GPU_STREAM_MINCOST, namespace mincost).
 //
 // There is no CPU fallback in this file: without a device every entry point
 // returns ENODEV.
@@ -503,6 +504,77 @@ parse_walk(const uint8_t* __restrict__ shard, const uint32_t* __restrict__ table
 }  // namespace parse
 
 // ---------------------------------------------------------------------------
+// min-cost parse (SQZ_GPU_STREAM_MINCOST, include/sqz_gpu.h): the table is rewritten so that every
+// word holds the chosen step -- (k << 16) | dist for a match of k <= len, 0 for a literal -- and the
+// greedy parse above then walks exactly the min-cost path.  Segments of kSegment positions at global
+// offsets that are multiples of kSegment; within one, backwards from its end e with c(j) = 0 for
+// j >= e,
+//   c(i) = min(8 + c(i + 1),  11 + len_extra(k) + pos_extra(dist) + c(i + k) for min_len <= k <= len)
+// ties to the longest step.  The extra-bit counts are those of symbols_of_match.
+// One warp per segment.  c(i) reads at most max_len <= 257 ahead, so the warp keeps the last
+// kRing costs in a shared ring, which starts as zeros: c beyond the segment's end.  At a match the
+// lanes share the lengths k and one redux.sync takes the minimum of (cost << 9) | (511 - k), which
+// breaks ties towards the larger k and ranks the literal (k = 1) after every match of equal cost;
+// costs stay below 2^18 (8 x 16384 for a segment of literals).  The table words of 32 positions come
+// in with one coalesced load and leave, rewritten, with one store; each position reads only its own.
+// ---------------------------------------------------------------------------
+namespace mincost {
+
+constexpr int kSegment = 16384;
+constexpr int kRing = 512;
+constexpr int kWarps = 4;        // segments per CTA
+
+__device__ __forceinline__ uint32_t len_extra_bits(uint32_t len) {     // 3 <= len <= 257
+    const uint32_t m = len - 3;
+    return m >= 8 ? 29u - (uint32_t)__clz((int)m) : 0u;
+}
+
+__device__ __forceinline__ uint32_t dist_extra_bits(uint32_t dist) {   // 1 <= dist <= 32767
+    const uint32_t q = dist - 1;
+    return q >= 4 ? 30u - (uint32_t)__clz((int)q) : 0u;
+}
+
+__global__ void __launch_bounds__(32 * kWarps)
+mincost_steps(uint32_t* __restrict__ table, size_t n, uint32_t min_len) {
+    __shared__ uint32_t ring_s[kWarps][kRing];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t s0 = ((size_t)blockIdx.x * kWarps + warp) * kSegment;
+    if (s0 >= n) { return; }                                   // the whole warp leaves together
+    const int size = (int)min((size_t)kSegment, n - s0);
+    uint32_t* ring = ring_s[warp];
+    for (int j = lane; j < kRing; j += 32) { ring[j] = 0; }
+    __syncwarp();
+    uint32_t after = 0;                                        // c(i + 1), the same in every lane
+    for (int base = (size - 1) & ~31; base >= 0; base -= 32) {
+        const int p = base + lane;
+        const uint32_t mine = p < size ? table[s0 + p] : 0u;
+        uint32_t out = 0;
+        for (int l = min(31, size - 1 - base); l >= 0; l--) {
+            const int i = base + l;
+            const uint32_t w = __shfl_sync(0xFFFFFFFFu, mine, l);
+            const uint32_t len = w >> 16;
+            uint32_t best = (after + 8) << 9 | (511u - 1u);    // the literal
+            if (len >= min_len) {
+                const uint32_t fixed = 11u + dist_extra_bits(w & 0xFFFF);
+                for (uint32_t k = min_len + lane; k <= len; k += 32) {
+                    const uint32_t c = fixed + len_extra_bits(k) + ring[(i + k) & (kRing - 1)];
+                    best = min(best, c << 9 | (511u - k));
+                }
+                best = __reduce_min_sync(0xFFFFFFFFu, best);
+            }
+            after = best >> 9;
+            const uint32_t k = 511u - (best & 511u);
+            if (lane == 0) { ring[i & (kRing - 1)] = after; }
+            if (lane == l) { out = k == 1 ? 0u : (k << 16 | (w & 0xFFFF)); }
+            __syncwarp();
+        }
+        if (p < size) { table[s0 + p] = out; }
+    }
+}
+
+}  // namespace mincost
+
+// ---------------------------------------------------------------------------
 // launchers (device-buffer ABI)
 // ---------------------------------------------------------------------------
 static int check_rules(uint32_t min_len, uint32_t max_len, uint32_t max_dist) {
@@ -513,25 +585,69 @@ static int check_rules(uint32_t min_len, uint32_t max_len, uint32_t max_dist) {
     return 0;
 }
 
-// --- optional CUDA-event timing of the match kernel (bench.py roofline leg) ---
+// --- optional CUDA-event timing of the match kernel (bench.py roofline leg) and of the min-cost steps ---
 static std::mutex g_time_mu;
 static bool g_timing = false;
-static std::vector<std::pair<cudaEvent_t, cudaEvent_t>> g_pending;
-static double g_match_seconds = 0;
-static uint64_t g_match_launches = 0;
 
-static void timing_drain_locked() {
-    for (auto& pr : g_pending) {
+struct KernelTimes {
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending;
+    double seconds = 0;
+    uint64_t launches = 0;
+};
+static KernelTimes g_match_times, g_mincost_times;
+
+static void timing_drain_locked(KernelTimes& t) {
+    for (auto& pr : t.pending) {
         float ms = 0;
         if (cudaEventSynchronize(pr.second) == cudaSuccess &&
             cudaEventElapsedTime(&ms, pr.first, pr.second) == cudaSuccess) {
-            g_match_seconds += 1e-3 * (double)ms;
-            g_match_launches++;
+            t.seconds += 1e-3 * (double)ms;
+            t.launches++;
         }
         cudaEventDestroy(pr.first);
         cudaEventDestroy(pr.second);
     }
-    g_pending.clear();
+    t.pending.clear();
+}
+
+// Events around one launcher call on stream s when timing is on: begin() records the start, end(ok)
+// the stop, and the pair waits in t.pending until the next query.  With timing off both do nothing.
+struct TimedLaunch {
+    KernelTimes& t;
+    cudaStream_t s;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    TimedLaunch(KernelTimes& times, cudaStream_t stream) : t(times), s(stream) {}
+    cudaError_t begin() {
+        {
+            std::lock_guard<std::mutex> lk(g_time_mu);
+            if (!g_timing) { return cudaSuccess; }
+            if (t.pending.size() > 4096) { timing_drain_locked(t); }
+        }
+        cudaError_t e = cudaEventCreate(&e0);
+        if (e == cudaSuccess) { e = cudaEventCreate(&e1); }
+        if (e == cudaSuccess) { e = cudaEventRecord(e0, s); }
+        return e;
+    }
+    void end(bool ok) {
+        if (ok && e0 != nullptr && e1 != nullptr && cudaEventRecord(e1, s) == cudaSuccess) {
+            std::lock_guard<std::mutex> lk(g_time_mu);
+            t.pending.emplace_back(e0, e1);
+        } else {
+            if (e0 != nullptr) { cudaEventDestroy(e0); }
+            if (e1 != nullptr) { cudaEventDestroy(e1); }
+        }
+        e0 = e1 = nullptr;
+    }
+    ~TimedLaunch() { end(false); }
+};
+
+static double kernel_seconds(KernelTimes& t, int reset, uint64_t* launches) {
+    std::lock_guard<std::mutex> lk(g_time_mu);
+    timing_drain_locked(t);
+    const double avg = t.launches ? t.seconds / (double)t.launches : 0.0;
+    if (launches != nullptr) { *launches = t.launches; }
+    if (reset) { t.seconds = 0; t.launches = 0; }
+    return avg;
 }
 
 extern "C" void sqz_gpu_set_timing(int on) {
@@ -540,12 +656,11 @@ extern "C" void sqz_gpu_set_timing(int on) {
 }
 
 extern "C" double sqz_gpu_match_kernel_seconds(int reset, uint64_t* launches) {
-    std::lock_guard<std::mutex> lk(g_time_mu);
-    timing_drain_locked();
-    const double avg = g_match_launches ? g_match_seconds / (double)g_match_launches : 0.0;
-    if (launches != nullptr) { *launches = g_match_launches; }
-    if (reset) { g_match_seconds = 0; g_match_launches = 0; }
-    return avg;
+    return kernel_seconds(g_match_times, reset, launches);
+}
+
+extern "C" double sqz_gpu_mincost_kernel_seconds(int reset, uint64_t* launches) {
+    return kernel_seconds(g_mincost_times, reset, launches);
 }
 
 static unsigned long long* g_tile_cycles = nullptr;   // debugging aid, see sqz_gpu_debug_tile_cycles
@@ -1008,33 +1123,15 @@ extern "C" int sqz_gpu_match_table_device_ws(const uint8_t* d_shard, size_t back
     if (n == 0) { return 0; }
     if (d_work == nullptr) { return fail(EINVAL, "null workspace"); }
     cudaStream_t s = (cudaStream_t)stream;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    bool timed = false;
-    {
-        std::lock_guard<std::mutex> lk(g_time_mu);
-        timed = g_timing;
-        if (timed && g_pending.size() > 4096) { timing_drain_locked(); }
-    }
-    if (timed) {
-        CU(cudaEventCreate(&e0));
-        CU(cudaEventCreate(&e1));
-        CU(cudaEventRecord(e0, s));
-    }
+    TimedLaunch timed(g_match_times, s);
+    CU(timed.begin());
     const int choice = g_kernel_choice;
     int r;
     const bool v2_ok = max_len > 32;      // the bit-sliced kernel measures runs in a 32-bit window
     if (choice != 1 && v2_ok && min_len == 3)      { r = launch_v2<3>(d_shard, back, n, ahead, max_len, max_dist, d_table, d_work, s); }
     else if (choice != 1 && v2_ok && min_len == 2) { r = launch_v2<2>(d_shard, back, n, ahead, max_len, max_dist, d_table, d_work, s); }
     else { r = launch_v1(d_shard, back, n, ahead, min_len, max_len, max_dist, d_table, s); }
-    if (timed) {
-        if (r == 0 && cudaEventRecord(e1, s) == cudaSuccess) {
-            std::lock_guard<std::mutex> lk(g_time_mu);
-            g_pending.emplace_back(e0, e1);
-        } else {
-            cudaEventDestroy(e0);
-            cudaEventDestroy(e1);
-        }
-    }
+    timed.end(r == 0);
     return r;
 }
 
@@ -1154,6 +1251,29 @@ static int check_flags(uint32_t flags, uint32_t allowed) {
     return 0;
 }
 
+// The min-cost parse prices matches with the buckets of the symbol words, so it exists within their
+// limits only, and it is a parse of its own: not together with the lazy rule.
+static int check_mincost(uint32_t flags, uint32_t min_len, uint32_t max_len, uint32_t max_dist) {
+    if ((flags & SQZ_GPU_STREAM_MINCOST) == 0) { return 0; }
+    if ((flags & SQZ_GPU_STREAM_LAZY) != 0) { return fail(EINVAL, "the min-cost and the lazy parse exclude each other"); }
+    return check_symbol_rules(min_len, max_len, max_dist);
+}
+
+// Rewrites d_table[0, n) into min-cost steps; the shard starts at a global offset that is a multiple
+// of mincost::kSegment.
+static int mincost_launch(uint32_t* d_table, size_t n, uint32_t min_len, cudaStream_t s) {
+    if (n == 0) { return 0; }
+    const size_t segments = (n + mincost::kSegment - 1) / mincost::kSegment;
+    const size_t ctas = (segments + mincost::kWarps - 1) / mincost::kWarps;
+    if (ctas > 0x7FFFFFFFull) { return fail(EINVAL, "shard too large for one launch"); }
+    TimedLaunch timed(g_mincost_times, s);
+    CU(timed.begin());
+    mincost::mincost_steps<<<(unsigned)ctas, 32 * mincost::kWarps, 0, s>>>(d_table, n, min_len);
+    LAUNCHED("mincost_steps");
+    timed.end(true);
+    return 0;
+}
+
 extern "C" int sqz_gpu_parse_device_ex(const uint8_t* d_shard, const uint32_t* d_table, size_t n,
                                        uint32_t entry, uint32_t min_len, uint32_t max_len, uint32_t flags,
                                        uint32_t* d_out, size_t out_cap, void* d_work,
@@ -1238,6 +1358,7 @@ struct sqz_gpu_stream {
     int kind = kConsumer;             // of its two stages: kTable, kTokens or kConsumer
     bool symbols = false;             // emit symbol words instead of plain tokens
     bool lazy = false;                // parse with the lazy rule
+    bool mincost = false;             // rewrite the table into min-cost steps before the parse
     Stage slot[2];
     const uint64_t* prev_result = nullptr;   // device: previous chunk's result (entry hand-off)
     cudaEvent_t prev_parsed = nullptr;
@@ -1313,6 +1434,11 @@ static int stream_launch_next(sqz_gpu_stream* st, uint16_t* len_out, uint16_t* d
     if (late != s.stream) { CU(cudaStreamWaitEvent(late, s.tabled, 0)); }
     if (st->kind != kTable) {
         const uint32_t* d_entry = nullptr;
+        // every chunk but the last holds whole segments (stream_open), so the chunk's segments are the
+        // input's, and the greedy parse of the rewritten table is the min-cost parse
+        if (st->mincost) {
+            if (int r = mincost_launch(s.d_table, n, st->min_len, late)) { return r; }
+        }
         if (st->prev_result != nullptr) {
             CU(cudaStreamWaitEvent(late, st->prev_parsed, 0));
             d_entry = reinterpret_cast<const uint32_t*>(st->prev_result + 1);  // low half of overshoot
@@ -1356,7 +1482,7 @@ static size_t default_chunk(size_t bytes, bool consumer) {
 
 static int stream_open(sqz_gpu_stream** out, int device, const uint8_t* data, size_t bytes,
                        uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
-                       size_t chunk, int kind, bool short_start = false) {
+                       size_t chunk, int kind, bool short_start = false, bool mincost = false) {
     *out = nullptr;
     if (int r = check_call(device, window, min_len, max_len, max_dist, data, bytes)) { return r; }
     sqz_gpu_stream* st = new (std::nothrow) sqz_gpu_stream();
@@ -1365,11 +1491,20 @@ static int stream_open(sqz_gpu_stream** out, int device, const uint8_t* data, si
     st->data = data;
     st->bytes = bytes;
     st->min_len = min_len; st->max_len = max_len; st->max_dist = max_dist;
+    st->mincost = mincost;
+    // The min-cost parse needs every chunk but the last to be whole segments.  The default chunks
+    // (2-32 MiB, 128 MiB) are; an explicit size and its short start are rounded up to them (a size
+    // too close to SIZE_MAX to round exceeds any input: its one chunk is the last).
+    auto whole_segments = [mincost](size_t b) {
+        const size_t seg = mincost::kSegment;
+        return mincost && b <= SIZE_MAX - seg ? (b + seg - 1) / seg * seg : b;
+    };
+    chunk = whole_segments(chunk);
     st->chunk = chunk ? chunk : default_chunk(bytes, kind == kConsumer);
     st->kind = kind;
     // token streams with the default chunking start with short chunks: 2, 4, 8, 16 MiB, then 32 MiB
     if (kind == kConsumer && chunk == 0 && st->chunk > ((size_t)2 << 20)) { st->ramp = (size_t)2 << 20; }
-    if (short_start && chunk >= ((size_t)4 << 20)) { st->ramp = chunk / 4; }
+    if (short_start && chunk >= ((size_t)4 << 20)) { st->ramp = whole_segments(chunk / 4); }
     const int slots = bytes > (st->ramp ? st->ramp : st->chunk) ? 2 : 1;
     for (int k = 0; k < slots && bytes > 0; k++) {
         if (int r = stage_take(st->slot[k], device, kind, st->chunk)) {
@@ -1394,15 +1529,18 @@ extern "C" int sqz_gpu_stream_open(sqz_gpu_stream** st, int device, const uint8_
                                    uint32_t max_len, uint32_t max_dist, size_t chunk_bytes,
                                    uint32_t flags) {
     if (st == nullptr) { return fail(EINVAL, "null stream handle"); }
-    if ((flags & ~(uint32_t)(SQZ_GPU_STREAM_SYMBOLS | SQZ_GPU_STREAM_SHORT_START | SQZ_GPU_STREAM_LAZY)) != 0) {
+    if ((flags & ~(uint32_t)(SQZ_GPU_STREAM_SYMBOLS | SQZ_GPU_STREAM_SHORT_START | SQZ_GPU_STREAM_LAZY |
+                             SQZ_GPU_STREAM_MINCOST)) != 0) {
         return fail(EINVAL, "unknown stream flags");
     }
     if (flags & SQZ_GPU_STREAM_SYMBOLS) {
         if (int r = check_symbol_rules(min_len, max_len, max_dist)) { return r; }
     }
+    if (int r = check_mincost(flags, min_len, max_len, max_dist)) { return r; }
     DeviceScope keep;
     if (int r = stream_open(st, device, data, bytes, window, min_len, max_len, max_dist,
-                            chunk_bytes, kConsumer, (flags & SQZ_GPU_STREAM_SHORT_START) != 0)) { return r; }
+                            chunk_bytes, kConsumer, (flags & SQZ_GPU_STREAM_SHORT_START) != 0,
+                            (flags & SQZ_GPU_STREAM_MINCOST) != 0)) { return r; }
     (*st)->symbols = (flags & SQZ_GPU_STREAM_SYMBOLS) != 0;
     (*st)->lazy = (flags & SQZ_GPU_STREAM_LAZY) != 0;
     if (bytes > 0) {
@@ -1458,16 +1596,19 @@ extern "C" void sqz_gpu_stream_close(sqz_gpu_stream* st) {
 // the caller's buffer, count x 4 bytes each (a pinned destination takes them by DMA while the next
 // chunk is searched; a pageable one through the driver's staging).  Nothing consumes the chunks
 // on the way, so the larger streaming chunk is used.  The lazy parse crosses its chunk seams as in the
-// token stream: every chunk searches its seam word.
+// token stream: every chunk searches its seam word.  The min-cost parse needs nothing across seams:
+// the 128 MiB chunks are whole segments.
 extern "C" int sqz_gpu_tokens_ex(const uint8_t* data, size_t bytes, uint32_t window,
                                  uint32_t min_len, uint32_t max_len, uint32_t max_dist, uint32_t flags,
                                  uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens) {
     if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
     *n_tokens = 0;
-    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY)) { return r; }
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY | SQZ_GPU_STREAM_MINCOST)) { return r; }
+    if (int r = check_mincost(flags, min_len, max_len, max_dist)) { return r; }
     sqz_gpu_stream* st = nullptr;
     DeviceScope keep;
-    if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kTokens)) {
+    if (int r = stream_open(&st, -1, data, bytes, window, min_len, max_len, max_dist, 0, kTokens, false,
+                            (flags & SQZ_GPU_STREAM_MINCOST) != 0)) {
         return r;
     }
     st->lazy = (flags & SQZ_GPU_STREAM_LAZY) != 0;
