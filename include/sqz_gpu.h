@@ -122,6 +122,29 @@ int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices,
                             uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
                             size_t* shard_tokens);
 
+/* sqz_gpu_tokens_multi_ex at shard boundaries of the caller's choice, and with
+ * the min-cost parse.  flags: 0, SQZ_GPU_STREAM_LAZY or SQZ_GPU_STREAM_MINCOST
+ * (within the bitstream's limits); any other bit or combination is EINVAL.
+ * cuts: n_devices - 1 non-decreasing global offsets, each <= bytes (shards may
+ * be empty); shard g is [cuts[g-1], cuts[g]) with cuts[-1] = 0 and
+ * cuts[n_devices-1] = bytes.  With SQZ_GPU_STREAM_MINCOST every cut is a
+ * multiple of 16384 or equal to bytes, so that every shard starts at a segment
+ * and all but the last hold whole segments; each shard then rewrites its own
+ * table into min-cost steps and nothing more crosses the seams than for the
+ * greedy parse.  cuts = NULL: the even cut, ceil(bytes / u) units of u bytes
+ * shared out as evenly as they go (the first ones one unit more), u = 1 without
+ * MINCOST (the cut of sqz_gpu_tokens_multi_ex), u = 16384 with it (the partial
+ * last segment in the last non-empty shard, shards past the segment count
+ * empty).  Every argument is checked before any device is touched; on EINVAL
+ * *n_tokens is 0.  The result is identical to sqz_gpu_tokens_ex() with the
+ * same flags for every valid cut list.                                       */
+int sqz_gpu_tokens_multi_cuts(const int* devices, int n_devices, const size_t* cuts /* n_devices - 1, or NULL */,
+                              const uint8_t* data, size_t bytes,
+                              uint32_t window, uint32_t min_len, uint32_t max_len,
+                              uint32_t max_dist, uint32_t flags,
+                              uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                              size_t* shard_tokens);
+
 /* Streaming form used by sqz_compress(): tokens arrive chunk by chunk, in
  * parse order, from double-buffered pinned memory while the device already
  * works on the next chunk.  *tokens stays valid until the next call.
@@ -158,8 +181,13 @@ int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices,
  * otherwise.  Every chunk but the last holds whole segments: the default
  * chunks already do, an explicit chunk_bytes (and its SHORT_START quarter) is
  * rounded up to a multiple of 16384.  sqz_gpu_tokens_ex takes the flag as
- * well; sqz_gpu_tokens_multi_ex and the device-buffer entry points do not yet
- * (EINVAL), because their shards are not cut at segment offsets.            */
+ * well, and so do the two calls made for shards: sqz_gpu_tokens_multi_cuts,
+ * which cuts at segment offsets, and sqz_gpu_mincost_steps_device, which
+ * rewrites one shard's table once before the flag-0 device-buffer parse.
+ * sqz_gpu_tokens_multi_ex keeps refusing it (EINVAL): its cut, sizes that
+ * differ by at most one byte, is not at segment offsets.  The device-buffer
+ * _ex calls refuse it too: they read the table without changing it, and the
+ * rewrite must run exactly once per table.                                   */
 typedef struct sqz_gpu_stream sqz_gpu_stream;
 #define SQZ_GPU_STREAM_SYMBOLS 1u       /* deliver symbol words instead of plain tokens */
 #define SQZ_GPU_STREAM_SHORT_START 2u   /* explicit chunk_bytes: start with chunk_bytes / 4, then / 2 */
@@ -253,6 +281,21 @@ int sqz_gpu_parse_device_ex(const uint8_t* d_shard, const uint32_t* d_table, siz
 int sqz_gpu_parse_exit_map_device_ex(const uint32_t* d_table, size_t n,
                                      uint32_t min_len, uint32_t max_len, uint32_t flags,
                                      void* d_work, uint16_t* d_exit_map, void* stream);
+
+/* The min-cost parse of a shard (SQZ_GPU_STREAM_MINCOST above): rewrites the
+ * n words of d_table, as sqz_gpu_match_table_device left them with the same
+ * rules, in place into min-cost steps -- (k << 16) | dist, or 0 for a literal.
+ * `first` is the shard's global offset, `bytes` the size of the whole input.
+ * After it, the flag-0 calls sqz_gpu_parse_exit_map_device(_ex) and
+ * sqz_gpu_parse_device(_ex) give the min-cost exit map and token stream (with
+ * SQZ_GPU_STREAM_SYMBOLS its symbol words), and the exit maps chain across
+ * shards as for the greedy parse.  Call it once per table: what it leaves are
+ * steps, not best matches, and a second rewrite would price those.  EINVAL
+ * unless first % 16384 == 0, first + n <= bytes, n % 16384 == 0 or
+ * first + n == bytes, and the rules are within the bitstream's limits
+ * (min_len >= 3, max_len <= 257, max_dist <= 32767).  n == 0 does nothing.   */
+int sqz_gpu_mincost_steps_device(uint32_t* d_table, size_t first, size_t n, size_t bytes,
+                                 uint32_t min_len, uint32_t max_len, uint32_t max_dist, void* stream);
 
 /* ---- one process per device ------------------------------------------------ *
  * Jobs that run one process per GPU (torchrun and the like) concatenate their

@@ -89,6 +89,9 @@ SYMBOLS = {
     "sqz_gpu_tokens_multi_ex": (C.c_int, [C.POINTER(C.c_int), C.c_int, u8p, size_t, C.c_uint32, C.c_uint32,
                                           C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, size_t, C.POINTER(size_t),
                                           C.POINTER(size_t)]),
+    "sqz_gpu_tokens_multi_cuts": (C.c_int, [C.POINTER(C.c_int), C.c_int, C.POINTER(size_t), u8p, size_t, C.c_uint32,
+                                            C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, size_t,
+                                            C.POINTER(size_t), C.POINTER(size_t)]),
     "sqz_gpu_stream_open": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, u8p, size_t, C.c_uint32, C.c_uint32,
                                       C.c_uint32, C.c_uint32, size_t, C.c_uint32]),
     "sqz_gpu_stream_next": (C.c_int, [C.c_void_p, C.POINTER(u32p), C.POINTER(size_t)]),
@@ -112,6 +115,8 @@ SYMBOLS = {
                                           C.c_uint32, C.c_void_p, size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sqz_gpu_parse_exit_map_device_ex": (C.c_int, [C.c_void_p, size_t, C.c_uint32, C.c_uint32, C.c_uint32,
                                                    C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sqz_gpu_mincost_steps_device": (C.c_int, [C.c_void_p, size_t, size_t, size_t, C.c_uint32, C.c_uint32,
+                                               C.c_uint32, C.c_void_p]),
     "sqz_gpu_device_alloc": (C.c_int, [C.POINTER(C.c_void_p), size_t]),
     "sqz_gpu_device_free": (None, [C.c_void_p]),
     "sqz_gpu_ipc_export": (C.c_int, [C.c_void_p, C.c_char_p]),

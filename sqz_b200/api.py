@@ -101,10 +101,15 @@ def tokens(data, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len: int 
 
 
 def tokens_multi(data, devices, window: int = 1 << 15, min_len: int = G1_MIN_LEN, max_len: int = G1_MAX_LEN,
-                 max_dist: int | None = None, return_shard_counts: bool = False, lazy: bool = False):
-    """The same token stream computed on several GPUs of this process (sqz_gpu_tokens_multi_ex):
-    contiguous shards with halos, seams chained on the host, token arrays concatenated in shard
-    order by copies sized by their counts.  Identical to tokens(lazy=lazy) for every device list."""
+                 max_dist: int | None = None, return_shard_counts: bool = False, lazy: bool = False,
+                 mincost: bool = False, cuts=None):
+    """The same token stream computed on several GPUs of this process: contiguous shards with halos, seams
+    chained on the host, token arrays concatenated in shard order by copies sized by their counts.
+    Identical to tokens(lazy=lazy, mincost=mincost) for every device list.  The default cut gives shards
+    whose sizes differ by at most one byte (sqz_gpu_tokens_multi_ex); mincost=True cuts at multiples of
+    16384 instead (shard.plan(..., align=shard.SEGMENT)), and `cuts` (len(devices) - 1 global offsets) sets
+    the shard boundaries -- both go through sqz_gpu_tokens_multi_cuts."""
+    flags = _parse_flags(lazy, mincost)
     L = _lib.load()
     d = _u8(data)
     w, lo, hi, md = _rules(window, min_len, max_len, max_dist)
@@ -112,9 +117,17 @@ def tokens_multi(data, devices, window: int = 1 << 15, min_len: int = G1_MIN_LEN
     out = np.empty(max(d.size, 1), dtype=np.uint32)
     n = C.c_size_t()
     per = (C.c_size_t * len(devices))()
-    rc = L.sqz_gpu_tokens_multi_ex(devs, len(devices), d.ctypes.data_as(u8p), d.size, w, lo, hi, md,
-                                   _lib.STREAM_LAZY if lazy else 0, out.ctypes.data, out.size, C.byref(n), per)
-    _check(rc, "sqz_gpu_tokens_multi_ex")
+    if mincost or cuts is not None:
+        if cuts is not None and len(cuts) != len(devices) - 1:
+            raise ValueError("cuts: len(devices) - 1 offsets")
+        at = None if cuts is None else (C.c_size_t * max(len(cuts), 1))(*[int(c) for c in cuts])
+        rc = L.sqz_gpu_tokens_multi_cuts(devs, len(devices), at, d.ctypes.data_as(u8p), d.size, w, lo, hi, md, flags,
+                                         out.ctypes.data, out.size, C.byref(n), per)
+        _check(rc, "sqz_gpu_tokens_multi_cuts")
+    else:
+        rc = L.sqz_gpu_tokens_multi_ex(devs, len(devices), d.ctypes.data_as(u8p), d.size, w, lo, hi, md, flags,
+                                       out.ctypes.data, out.size, C.byref(n), per)
+        _check(rc, "sqz_gpu_tokens_multi_ex")
     t = out[: n.value].copy()
     return (t, [int(x) for x in per]) if return_shard_counts else t
 

@@ -1325,6 +1325,19 @@ extern "C" int sqz_gpu_parse_exit_map_device(const uint32_t* d_table, size_t n,
     return sqz_gpu_parse_exit_map_device_ex(d_table, n, min_len, max_len, 0, d_work, d_exit_map, stream);
 }
 
+// A shard's segments are the input's when it starts at a multiple of the segment and holds whole
+// segments, or runs to the end of the input.
+extern "C" int sqz_gpu_mincost_steps_device(uint32_t* d_table, size_t first, size_t n, size_t bytes,
+                                            uint32_t min_len, uint32_t max_len, uint32_t max_dist, void* stream) {
+    if (int r = check_rules(min_len, max_len, max_dist)) { return r; }
+    if (int r = check_symbol_rules(min_len, max_len, max_dist)) { return r; }
+    if (first % mincost::kSegment != 0 || first > bytes || n > bytes - first ||
+        (n % mincost::kSegment != 0 && first + n != bytes)) {
+        return fail(EINVAL, "a min-cost shard starts at a multiple of 16384 and holds whole segments or ends at bytes");
+    }
+    return mincost_launch(d_table, n, min_len, (cudaStream_t)stream);
+}
+
 // ---------------------------------------------------------------------------
 // host-buffer ABI: chunked, double-buffered pipeline
 // ---------------------------------------------------------------------------
@@ -1690,17 +1703,34 @@ extern "C" int sqz_gpu_match_table(const uint8_t* data, size_t bytes, uint32_t w
 // their counts: device -> host when tokens_out is host memory, peer-to-peer (cudaMemcpyPeerAsync
 // over NVLink) when it is device memory.  The lazy parse adds one dependency per seam, the best match
 // at the next shard's first position (table[n]), which every shard searches from its own halos: no
-// exchange beyond the exit maps.
+// exchange beyond the exit maps.  The min-cost parse adds none: with every shard starting at a multiple
+// of mincost::kSegment and holding whole segments (all but the last), a shard's segments are the input's,
+// and each shard rewrites its own table before its exit map.
 // ---------------------------------------------------------------------------
-static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_t* data, size_t bytes,
-                     uint32_t min_len, uint32_t max_len, uint32_t max_dist, bool lazy, uint32_t* tokens_out,
-                     size_t tokens_cap, bool out_on_device, int out_device, size_t* n_tokens,
-                     size_t* shard_tokens) {
-    // phase A on every device at once: upload, match table (and the seam word), composed exit map
-    const size_t base = bytes / parts.size(), extra = bytes % parts.size();
-    size_t first = 0;
+
+// The shard boundaries of [0, bytes) cut into n shards of whole units: ceil(bytes / unit) units shared
+// out as evenly as they go, the first (units % n) shards one unit more, every boundary clamped to bytes
+// (so the partial last unit lives in the last non-empty shard, and shards past the units are empty).
+// Returns n + 1 offsets, from 0 to bytes.  unit = 1 gives shards whose sizes differ by at most one byte.
+static std::vector<size_t> even_cuts(size_t bytes, size_t n, size_t unit) {
+    const size_t units = (bytes + unit - 1) / unit, base = units / n, extra = units % n;
+    std::vector<size_t> at(n + 1, 0);
+    for (size_t g = 0; g < n; g++) {
+        at[g + 1] = std::min(bytes, at[g] + (base + (g < extra ? 1 : 0)) * unit);
+    }
+    return at;
+}
+
+// `at`: parts.size() + 1 non-decreasing shard boundaries from 0 to bytes.  `mincost` needs every
+// boundary at a multiple of mincost::kSegment or at bytes.
+static int multi_run(std::vector<Stage>& parts, const int* devices, const std::vector<size_t>& at,
+                     const uint8_t* data, size_t bytes, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                     bool lazy, bool mincost, uint32_t* tokens_out, size_t tokens_cap, bool out_on_device,
+                     int out_device, size_t* n_tokens, size_t* shard_tokens) {
+    // phase A on every device at once: upload, match table (and the seam word or the min-cost steps),
+    // composed exit map
     for (size_t g = 0; g < parts.size(); g++) {
-        const size_t n = base + (g < extra ? 1 : 0);
+        const size_t first = at[g], n = at[g + 1] - at[g];
         if (n > 0) {
             Stage& p = parts[g];
             CU(cudaSetDevice(devices[g]));
@@ -1711,12 +1741,14 @@ static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_
                 if (int r = seam_word(p.d_data + back, back, n, ahead, min_len, max_len, max_dist, p.d_table,
                                       p.stream)) { return r; }
             }
+            if (mincost) {
+                if (int r = mincost_launch(p.d_table, n, min_len, p.stream)) { return r; }
+            }
             if (int r = sqz_gpu_parse_exit_map_device_ex(p.d_table, n, min_len, max_len, lazy ? SQZ_GPU_STREAM_LAZY : 0,
                                                          p.d_work, p.d_map, p.stream)) { return r; }
             CU(cudaMemcpyAsync(p.h_map, p.d_map, (size_t)max_len * 2, cudaMemcpyDeviceToHost, p.stream));
             CU(cudaEventRecord(p.tabled, p.stream));
         }
-        first += n;
     }
     // seams: shard g+1 is entered where shard g's last token ends
     uint32_t entry = 0;
@@ -1759,14 +1791,12 @@ static int multi_run(std::vector<Stage>& parts, const int* devices, const uint8_
     return total > tokens_cap ? fail(E2BIG, "token buffer too small") : 0;
 }
 
-extern "C" int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices, const uint8_t* data, size_t bytes,
-                                       uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
-                                       uint32_t flags, uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
-                                       size_t* shard_tokens) {
-    if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
-    *n_tokens = 0;
-    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY)) { return r; }
-    if (devices == nullptr || n_devices < 1 || n_devices > kMaxDevices) { return fail(EINVAL, "bad device list"); }
+// The multi-device calls after their own argument checks: `at` holds the shard boundaries, flags are
+// 0, LAZY or MINCOST.
+static int multi_call(const int* devices, int n_devices, const std::vector<size_t>& at, const uint8_t* data,
+                      size_t bytes, uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                      uint32_t flags, uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                      size_t* shard_tokens) {
     DeviceScope keep;
     int device = devices[0];
     if (int r = check_call(device, window, min_len, max_len, max_dist, data, bytes)) { return r; }
@@ -1800,10 +1830,55 @@ extern "C" int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices, const 
         }
     }
     std::vector<Stage> parts((size_t)n_devices);
-    int rc = multi_run(parts, devices, data, bytes, min_len, max_len, max_dist, (flags & SQZ_GPU_STREAM_LAZY) != 0,
-                       tokens_out, tokens_cap, out_on_device, out_device, n_tokens, shard_tokens);
+    int rc = multi_run(parts, devices, at, data, bytes, min_len, max_len, max_dist, (flags & SQZ_GPU_STREAM_LAZY) != 0,
+                       (flags & SQZ_GPU_STREAM_MINCOST) != 0, tokens_out, tokens_cap, out_on_device, out_device,
+                       n_tokens, shard_tokens);
     for (Stage& p : parts) { rc = stage_finish(p, rc); }
     return rc;
+}
+
+static int check_device_list(const int* devices, int n_devices) {
+    if (devices == nullptr || n_devices < 1 || n_devices > kMaxDevices) { return fail(EINVAL, "bad device list"); }
+    return 0;
+}
+
+extern "C" int sqz_gpu_tokens_multi_ex(const int* devices, int n_devices, const uint8_t* data, size_t bytes,
+                                       uint32_t window, uint32_t min_len, uint32_t max_len, uint32_t max_dist,
+                                       uint32_t flags, uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                                       size_t* shard_tokens) {
+    if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
+    *n_tokens = 0;
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY)) { return r; }
+    if (int r = check_device_list(devices, n_devices)) { return r; }
+    return multi_call(devices, n_devices, even_cuts(bytes, (size_t)n_devices, 1), data, bytes, window, min_len,
+                      max_len, max_dist, flags, tokens_out, tokens_cap, n_tokens, shard_tokens);
+}
+
+extern "C" int sqz_gpu_tokens_multi_cuts(const int* devices, int n_devices, const size_t* cuts,
+                                         const uint8_t* data, size_t bytes, uint32_t window, uint32_t min_len,
+                                         uint32_t max_len, uint32_t max_dist, uint32_t flags,
+                                         uint32_t* tokens_out, size_t tokens_cap, size_t* n_tokens,
+                                         size_t* shard_tokens) {
+    if (n_tokens == nullptr) { return fail(EINVAL, "null n_tokens"); }
+    *n_tokens = 0;
+    if (int r = check_flags(flags, SQZ_GPU_STREAM_LAZY | SQZ_GPU_STREAM_MINCOST)) { return r; }
+    if (int r = check_mincost(flags, min_len, max_len, max_dist)) { return r; }
+    if (int r = check_device_list(devices, n_devices)) { return r; }
+    const bool mincost = (flags & SQZ_GPU_STREAM_MINCOST) != 0;
+    const size_t unit = mincost ? (size_t)mincost::kSegment : 1;
+    std::vector<size_t> at = even_cuts(bytes, (size_t)n_devices, unit);
+    if (cuts != nullptr) {
+        for (int g = 1; g < n_devices; g++) {
+            const size_t c = cuts[g - 1];
+            if (c < at[g - 1] || c > bytes) { return fail(EINVAL, "cuts must be non-decreasing and <= bytes"); }
+            if (c % unit != 0 && c != bytes) {
+                return fail(EINVAL, "the min-cost parse needs every cut at a multiple of 16384 or at bytes");
+            }
+            at[g] = c;
+        }
+    }
+    return multi_call(devices, n_devices, at, data, bytes, window, min_len, max_len, max_dist, flags, tokens_out,
+                      tokens_cap, n_tokens, shard_tokens);
 }
 
 extern "C" int sqz_gpu_tokens_multi(const int* devices, int n_devices, const uint8_t* data, size_t bytes,

@@ -66,6 +66,20 @@ def exit_map(table: torch.Tensor, n: int, min_len: int = G1_MIN_LEN, max_len: in
     return out
 
 
+def mincost_steps(table: torch.Tensor, first: int, n: int, total: int, min_len: int = G1_MIN_LEN,
+                  max_len: int = G1_MAX_LEN, max_dist: int = (1 << 15) - 1) -> torch.Tensor:
+    """Rewrites a shard's n table words (match_table with the same rules) in place into min-cost steps and
+    returns the table; exit_map and parse (greedy, the default) of it then give the min-cost parse.  `first`
+    is the shard's global offset, `total` the whole input's size: the shard starts at a multiple of 16384
+    and holds whole segments or ends at `total` (shard.plan(..., align=shard.SEGMENT)).  Once per table
+    (sqz_gpu_mincost_steps_device)."""
+    L = _lib.load()
+    _need(table, "table", torch.int32, n, table.device if isinstance(table, torch.Tensor) else None)
+    rc = L.sqz_gpu_mincost_steps_device(table.data_ptr(), first, n, total, min_len, max_len, max_dist, _stream())
+    _check(rc, "sqz_gpu_mincost_steps_device")
+    return table
+
+
 def parse(buf: torch.Tensor, first: int, table: torch.Tensor, n: int, entry: int = 0, min_len: int = G1_MIN_LEN,
           max_len: int = G1_MAX_LEN, symbols: bool = False, lazy: bool = False):
     """Greedy (squeeze.h:337,377-394; the default) or lazy parse of one shard: (tokens int32[count], overshoot).

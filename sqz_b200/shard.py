@@ -8,11 +8,16 @@ overshoot of shard g's last token.  Every shard publishes exit_map[e] = "oversho
 produce when entered at offset e" (sqz_gpu_parse_exit_map_device); chaining those maps
 gives every shard its true entry after one tiny all-gather.
 
-Nothing here depends on the parse rule.  The lazy parse steps 1 or len <= max_len as well, so
-entries and overshoots keep their bounds; its one extra input at a seam, the best match at the
-next shard's first position, every shard searches itself from its own look-ahead halo
-(device.match_table(..., seam=True)), and its maps (device.exit_map(..., lazy=True)) chain here
-unchanged.
+The lazy parse steps 1 or len <= max_len as well, so entries and overshoots keep their bounds;
+its one extra input at a seam, the best match at the next shard's first position, every shard
+searches itself from its own look-ahead halo (device.match_table(..., seam=True)), and its maps
+(device.exit_map(..., lazy=True)) chain here unchanged.
+
+The min-cost parse is the one rule the cut matters to: its steps depend on the table words of
+their own 16384-position segment, at global offsets that are multiples of 16384, so every shard
+has to start at a segment and hold whole ones (all but the last): plan(..., align=SEGMENT).  Each
+shard then rewrites its own table (device.mincost_steps) and the greedy exit maps and parse of the
+rewritten table chain here unchanged, with no extra input at the seams.
 """
 from __future__ import annotations
 
@@ -20,6 +25,8 @@ from dataclasses import dataclass
 from typing import Sequence
 
 import numpy as np
+
+SEGMENT = 16384     # positions of a min-cost segment (include/sqz_gpu.h, SQZ_GPU_STREAM_MINCOST)
 
 
 @dataclass(frozen=True)
@@ -41,14 +48,19 @@ class Shard:
         return self.first + self.n + self.ahead
 
 
-def plan(total: int, world: int, max_dist: int, max_len: int) -> list[Shard]:
-    """Cut [0, total) into `world` contiguous shards of (almost) equal size."""
+def plan(total: int, world: int, max_dist: int, max_len: int, *, align: int = 1) -> list[Shard]:
+    """Cut [0, total) into `world` contiguous shards of whole `align`-byte units: ceil(total / align) units
+    shared out as evenly as they go (the first ones one unit more), every cut clamped to `total`.  align=1:
+    sizes differ by at most one byte (the cut of sqz_gpu_tokens_multi_ex); align=SEGMENT: the cut of the
+    min-cost parse, the partial last segment in the last non-empty shard, shards past the segments empty."""
     if world < 1:
         raise ValueError("world must be >= 1")
-    base, extra = divmod(total, world)
+    if align < 1:
+        raise ValueError("align must be >= 1")
+    base, extra = divmod(-(-total // align), world)
     out, first = [], 0
     for r in range(world):
-        n = base + (1 if r < extra else 0)
+        n = min(total, first + (base + (1 if r < extra else 0)) * align) - first
         out.append(Shard(r, first, n, min(first, max_dist), min(total - (first + n), max_len)))
         first += n
     return out
