@@ -751,9 +751,6 @@ struct ScopedEvent {
 // ---------------------------------------------------------------------------
 constexpr size_t kCursorBytes = 256;
 
-// Distance slices of a small shard (match_bitsliced.cuh): as many as it takes to give the device
-// about four waves of CTAs, a power of two, at most 32; none once the tiles alone fill it.
-// Fixed numbers (444 resident CTAs: 148 SMs x 3), so that the workspace size depends on n only.
 struct SlicePlan { int q; int slices; int slice_words; size_t stride; };
 
 // How a shard is cut (match_bitsliced.cuh).  From a wave of throughput tiles on (444 resident CTAs of

@@ -6,6 +6,7 @@ import pytest
 
 import sqz_b200 as sq
 from sqz_b200 import corpus, shard
+from match_inputs import far_repeat_input
 
 pytestmark = pytest.mark.gpu
 
@@ -303,40 +304,12 @@ def test_randomised_inputs_and_rules(seed, oracle, kernel):
     assert end == n and t.size == ot.size and (t == ot).all()
 
 
-def _far_repeat_input(rng, n):
-    """Blocks of 4-12 KiB repeated at distances of 30,000-32,767 with a few defects, runs of 32
-    spaces and of one byte value in between: the far max_len early-out (squeeze.h:353) next to
-    thousands of near candidates that tie on their first bytes."""
-    out = []
-    size = 0
-    words = [b"    " * 8, b"\t\t", b"static ", b"const ", b"uint32_t ", b"return ", b";\n", b"if (", b") {\n", b"}\n"]
-    def filler(k):
-        parts, got = [], 0
-        while got < k:
-            w = words[int(rng.integers(0, len(words)))] if rng.random() < 0.7 else bytes(rng.integers(97, 123, int(rng.integers(1, 9)), dtype=np.uint8))
-            parts.append(w); got += len(w)
-        return np.frombuffer(b"".join(parts)[:k], np.uint8)
-    while size < n:
-        block = filler(int(rng.integers(4096, 12288)))
-        gap = int(rng.integers(30000, 32768)) - block.size
-        mid = filler(max(gap, 1)).copy()
-        if rng.random() < 0.5:
-            at = int(rng.integers(0, max(mid.size - 600, 1)))
-            mid[at:at + int(rng.integers(33, 600))] = 32 if rng.random() < 0.5 else 0
-        again = block.copy()
-        for at in rng.integers(0, block.size, int(rng.integers(0, 4))).tolist():
-            again[at] ^= 1
-        out += [block, mid, again]
-        size += 2 * block.size + mid.size
-    return np.concatenate(out)[:n].copy()
-
-
 @pytest.mark.parametrize("seed", range(6))
 def test_far_repeats_fuzz(seed, oracle, kernel):
     """Full table == oracle B on far-repeat inputs, == the brute-force loop on sampled positions."""
     rng = np.random.default_rng(7000 + seed)
     n = int(rng.choice([90000, 200000, 400000]))
-    d = _far_repeat_input(rng, n)
+    d = far_repeat_input(rng, n)
     ln, ds = sq.match_table(d, 1 << 15)
     oln, ods = oracle.match_table(d, 1 << 15, fast=True)
     bad = np.nonzero((ln != oln) | (ds != ods))[0]
@@ -353,7 +326,7 @@ def test_far_repeats_fuzz(seed, oracle, kernel):
 def test_capped_inheritance_other_caps(mx, md, oracle):
     """The far-repeat shortcut of phase 2 depends on max_len (its slack shrinks to max_len - 32)."""
     rng = np.random.default_rng(mx * 7 + md)
-    d = _far_repeat_input(rng, 150000)
+    d = far_repeat_input(rng, 150000)
     window = 1 << 16 if md > 32767 else 1 << 15
     ln, ds = sq.match_table(d, window, 3, mx, md)
     oln, ods = oracle.match_table(d, window, fast=True, min_len=3, max_len=mx, max_dist=md)
@@ -440,8 +413,8 @@ def test_tokens_multi_bad_arguments():
 
 @pytest.mark.parametrize("mib,offset", [(7.3, 0), (9, 1 << 20), (11.5, 3276897)])
 def test_shards_of_a_few_waves(mib, offset, oracle):
-    """Between one and a few waves of tiles the last, partial wave is cut into distance slices as well
-    (sqz_gpu.cu: launch_tiles): full table == oracle B, with and without a look-back halo."""
+    """Between one and a few waves of tiles (7.3-11.5 MiB): the unsliced throughput shape (sqz_gpu.cu:
+    slice_plan), partial last wave included: full table == oracle B, with and without a look-back halo."""
     from sqz_b200 import device
     n = int(mib * (1 << 20))
     d = corpus.synthetic(n, offset)
