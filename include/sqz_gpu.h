@@ -147,7 +147,11 @@ int sqz_gpu_tokens_multi_cuts(const int* devices, int n_devices, const size_t* c
 
 /* Streaming form used by sqz_compress(): tokens arrive chunk by chunk, in
  * parse order, from double-buffered pinned memory while the device already
- * works on the next chunk.  *tokens stays valid until the next call.
+ * works on the next chunk.  *tokens stays valid until the next call.  *count
+ * is 0 only when every token has been delivered; later calls return 0 again.
+ * A chunk that lies inside the previous chunk's last match (possible when
+ * chunk_bytes < max_len) is delivered together with the next one.  A chunk
+ * larger than the input is the input: the staging is sized by the input.
  * chunk_bytes = 0: chunks of 2, 4, 8, 16, then 32 MiB -- a consumer slower
  * than the search starts after milliseconds.  chunk_bytes > 0: chunks of that
  * size -- for a consumer faster than the search, which only has to keep the

@@ -915,6 +915,9 @@ constexpr size_t kParkBytes = (size_t)12 << 30;
 
 // a stage of this kind for n positions on `device`, which is the current device
 static int stage_take(Stage& s, int device, int kind, size_t n) {
+    // no device holds 2^60 positions, and beyond them the power of two below and the stage's byte counts
+    // (several bytes per position) would overflow
+    if (n > ((size_t)1 << 60)) { return fail(ENOMEM, "staging for more than 2^60 positions"); }
     size_t cap = (size_t)1 << 20;            // a power of two (>= 1 Mi) so that calls of similar size share stages
     while (cap < n) { cap <<= 1; }
     {
@@ -1516,8 +1519,9 @@ static int stream_open(sqz_gpu_stream** out, int device, const uint8_t* data, si
     if (kind == kConsumer && chunk == 0 && st->chunk > ((size_t)2 << 20)) { st->ramp = (size_t)2 << 20; }
     if (short_start && chunk >= ((size_t)4 << 20)) { st->ramp = whole_segments(chunk / 4); }
     const int slots = bytes > (st->ramp ? st->ramp : st->chunk) ? 2 : 1;
+    // no chunk is larger than the input, however large the size asked for
     for (int k = 0; k < slots && bytes > 0; k++) {
-        if (int r = stage_take(st->slot[k], device, kind, st->chunk)) {
+        if (int r = stage_take(st->slot[k], device, kind, std::min(st->chunk, bytes))) {
             sqz_gpu_stream_close(st);
             return r;
         }
@@ -1572,27 +1576,33 @@ extern "C" int sqz_gpu_stream_next(sqz_gpu_stream* st, const uint32_t** tokens, 
     CU(cudaSetDevice(st->device));
     // keep the device busy: the slot the caller has just finished reading is free now
     static const bool trace = getenv("SQZ_TRACE") != nullptr;
-    const auto t0 = std::chrono::steady_clock::now();
-    if (st->launched < st->bytes) {
-        if (int r = stream_launch_next(st, nullptr, nullptr)) { return r; }
+    // A chunk that lies inside the previous chunk's last match (chunk_bytes < max_len) has no tokens:
+    // it is consumed here and the next one read, so that a count of 0 only ever means the end.
+    for (;;) {
+        const auto t0 = std::chrono::steady_clock::now();
+        if (st->launched < st->bytes) {
+            if (int r = stream_launch_next(st, nullptr, nullptr)) { return r; }
+        }
+        const auto t1 = std::chrono::steady_clock::now();
+        Stage& s = st->slot[st->read_slot];
+        CU(cudaEventSynchronize(s.done));
+        if (trace) {
+            const auto t2 = std::chrono::steady_clock::now();
+            fprintf(stderr, "sqz_gpu_stream_next: queued the next chunk in %.1f ms, waited %.1f ms for this one\n",
+                    std::chrono::duration<double, std::milli>(t1 - t0).count(),
+                    std::chrono::duration<double, std::milli>(t2 - t1).count());
+        }
+        const uint64_t n_tok = s.h_result[0];
+        if (n_tok > s.n) { return fail(EIO, "parse produced more tokens than positions"); }
+        s.busy = false;
+        st->delivered = s.first + s.n;
+        st->read_slot ^= 1;
+        if (n_tok != 0 || st->delivered >= st->bytes) {
+            *tokens = s.h_tokens;
+            *count = (size_t)n_tok;
+            return 0;
+        }
     }
-    const auto t1 = std::chrono::steady_clock::now();
-    Stage& s = st->slot[st->read_slot];
-    CU(cudaEventSynchronize(s.done));
-    if (trace) {
-        const auto t2 = std::chrono::steady_clock::now();
-        fprintf(stderr, "sqz_gpu_stream_next: queued the next chunk in %.1f ms, waited %.1f ms for this one\n",
-                std::chrono::duration<double, std::milli>(t1 - t0).count(),
-                std::chrono::duration<double, std::milli>(t2 - t1).count());
-    }
-    const uint64_t n_tok = s.h_result[0];
-    if (n_tok > s.n) { return fail(EIO, "parse produced more tokens than positions"); }
-    s.busy = false;
-    st->delivered = s.first + s.n;
-    st->read_slot ^= 1;
-    *tokens = s.h_tokens;
-    *count = (size_t)n_tok;
-    return 0;
 }
 
 extern "C" void sqz_gpu_stream_close(sqz_gpu_stream* st) {
